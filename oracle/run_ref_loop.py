@@ -6,7 +6,7 @@
                     (`cuda` if available, fno/train.py:32) -- on the GPU box this is "the reference on the same B200"
 --model dropin    : `fno.fno` / `fno_aux.fno_aux` are shadowed in sys.modules by fno_b200.fno / fno_b200.fno_aux before the
                     loop is imported (INTEGRATION.md): the loop itself is untouched and drives the sm_100a kernels
-The reference files are taken from /root/reference (build container) or oracle/_ref/ (GPU box; oracle/build_ref.py).
+The reference files are taken from oracle/_ref/ (oracle/build_ref.py).
 Recipe of SURVEY.md appendix B: stub h5py / matplotlib, register the synthetic datasets under the loader module names, disable
 wandb, call run_training(**kwargs).  TEST INFRASTRUCTURE ONLY.
 """
@@ -36,10 +36,11 @@ DEFAULT_CFG = {
 
 
 def ref_root() -> Path:
-    for cand in (Path("/root/reference/pdebench/models"), ROOT / "oracle" / "_ref"):
-        if (cand / "fno" / "train.py").exists():
-            return cand
-    raise SystemExit("reference files not found: run `python oracle/build_ref.py` in the build container")
+    ref = ROOT / "oracle" / "_ref"
+    if not (ref / "fno" / "train.py").exists():
+        raise SystemExit("reference files not found: build() with PDEBENCH_MODELS=<pdebench>/pdebench/models, or "
+                         "python oracle/build_ref.py <pdebench>/pdebench/models")
+    return ref
 
 
 def main():

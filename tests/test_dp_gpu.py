@@ -4,7 +4,7 @@
 * the CUDA-graph step (two graphs around inline bucket all-reduces) == the eager step with hook-issued, overlapped
   all-reduces, parameter for parameter, after several optimizer steps;
 * a ragged global batch (unequal local batches, fno_b200.data.epoch_plan weights) still gives the global-mean gradient.
-Skipped on a single-GPU box (the driver's `-m gpu` tier); run with `gpurun --gpus 2 -- python -m pytest tests/test_dp_gpu.py`.
+Skipped on a machine with fewer than two GPUs.
 """
 import os
 import socket
@@ -92,7 +92,7 @@ def _worker(rank, world, port, out_dir):
 @pytest.mark.timeout(240)
 def test_two_gpu_data_parallel_step(tmp_path):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     mp.spawn(_worker, args=(2, _free_port(), str(tmp_path)), nprocs=2, join=True)
     res = torch.load(tmp_path / "dp_gpu.pt")
     print(res)
