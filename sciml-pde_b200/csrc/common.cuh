@@ -158,6 +158,43 @@ __device__ __forceinline__ float gelu_fast_grad(float s) {
   return fmaf(s * 0.3989422804014327f, e, cdf);
 }
 
+// Two-element forms on the packed f32x2 pipe (FFMA2 / FMUL2 / FADD2): every lane is rounded exactly like the scalar
+// instruction and the operations run in the scalar forms' order, so .x / .y are bit-identical to gelu_fast /
+// gelu_fast_both of .x / .y, at one issue slot per two elements.  The epilogues that use them are bound by
+// instruction issue, not by the FMA pipe.  Written on nas = -|s|: u = nas c gives the same u^2, fma(-c, nas, 1) the
+// same 1 + c|s|, and fma(nas, q, max(s, 0)) is the scalar fma(-|s|, q, max(s, 0)); 0.5 - q is fma(q, -1, 0.5).
+__device__ __forceinline__ float2 f32x2(float a) { return make_float2(a, a); }
+__device__ __forceinline__ float2 gelu_half_erfc2(float2 nas, float2& e) {
+  const float2 u = __fmul2_rn(nas, f32x2(0.8493218002880191f));
+  const float2 d = __ffma2_rn(f32x2(-0.2316418882663604f), nas, f32x2(1.0f));
+  const float2 uu = __fmul2_rn(u, u);
+  float2 t;
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(t.x) : "f"(d.x));
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(t.y) : "f"(d.y));
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e.x) : "f"(-uu.x));
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e.y) : "f"(-uu.y));
+  float2 poly = __ffma2_rn(f32x2(0.5307027145f), t, f32x2(-0.7265760135f));
+  poly = __ffma2_rn(poly, t, f32x2(0.7107068705f));
+  poly = __ffma2_rn(poly, t, f32x2(-0.142248368f));
+  poly = __ffma2_rn(poly, t, f32x2(0.127414796f));
+  return __fmul2_rn(__fmul2_rn(poly, t), e);
+}
+__device__ __forceinline__ float2 gelu_fast2(float2 s) {
+  float2 e;
+  const float2 nas = make_float2(-fabsf(s.x), -fabsf(s.y));
+  const float2 q = gelu_half_erfc2(nas, e);
+  return __ffma2_rn(nas, q, make_float2(fmaxf(s.x, 0.0f), fmaxf(s.y, 0.0f)));
+}
+__device__ __forceinline__ void gelu_fast_both2(float2 s, float2& g, float2& gp) {
+  float2 e;
+  const float2 nas = make_float2(-fabsf(s.x), -fabsf(s.y));
+  const float2 q = gelu_half_erfc2(nas, e);
+  g = __ffma2_rn(nas, q, make_float2(fmaxf(s.x, 0.0f), fmaxf(s.y, 0.0f)));
+  const float2 r = __ffma2_rn(q, f32x2(-1.0f), f32x2(0.5f));
+  const float2 cdf = __fadd2_rn(f32x2(0.5f), make_float2(copysignf(r.x, s.x), copysignf(r.y, s.y)));
+  gp = __ffma2_rn(__fmul2_rn(s, f32x2(0.3989422804014327f)), e, cdf);
+}
+
 // ---- mbarrier / bulk-copy (TMA, 1-D) helpers --------------------------------------------------
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {

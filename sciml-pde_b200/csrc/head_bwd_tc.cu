@@ -53,7 +53,7 @@ constexpr int B3_LBO = 144, B3_SBO = 16 * B3_LBO, B3_BYTES = 4 * B3_SBO;   // h^
 constexpr int A2_LBO = 144, A2_SBO = 32 * A2_LBO, A2_BYTES = 8 * A2_SBO;   // dpre [px 64][j 128]
 constexpr int GT_BYTES = 2 * BT_PX * BT_GV * 4;                     // dout * std, two slots
 constexpr int BT_OPER_BYTES = 2 * (AW1_BYTES + B2_BYTES + 2 * BH_BYTES + 2 * B3_BYTES + A2_BYTES) + GT_BYTES;
-constexpr int BT_NBARS = 16;
+constexpr int BT_NBARS = 17;
 constexpr int BT_SMEM = BT_OPER_BYTES + BT_NBARS * 8 + 16;
 
 // TMEM columns (512 allocated: the CTA owns its SM)
@@ -97,17 +97,18 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
   unsigned char* b3_lo = b3_hi + 2 * B3_BYTES;
   unsigned char* a2_hi = b3_lo + 2 * B3_BYTES;
   unsigned char* a2_lo = a2_hi + A2_BYTES;
-  float4* gt = reinterpret_cast<float4*>(a2_lo + A2_BYTES);          // [2][64] dout * std
+  float4* gt = reinterpret_cast<float4*>(a2_lo + A2_BYTES);          // [2][32 pixel pairs][8 variables][2] dout * std
   unsigned long long* bars = reinterpret_cast<unsigned long long*>(bsm + BT_OPER_BYTES);
   unsigned long long* bh_ready = bars;        // [2] loaders -> MMA, epilogue: h tile (a) + dout tile staged
   unsigned long long* bh_free = bars + 2;     // [2] MMA (a) done -> loaders
   unsigned long long* b3_ready = bars + 4;    // [2] loaders -> MMA: h^T tile staged for (c)
-  unsigned long long* d2_full = bars + 6;     // [2] MMA (b), (c) done: dh accumulator full, h^T slot free
+  unsigned long long* d2_full = bars + 6;     // [2] MMA (b), (c) done: h^T slot free
   unsigned long long* d2_free = bars + 8;     // [2] dh accumulator drained
   unsigned long long* g_free = bars + 10;     // [2] dout tile consumed by the epilogue
   unsigned long long* d1_full = bars + 12;    // [2] MMA (a) done: pre^T ready
   unsigned long long* a23_ready = bars + 14;  // epilogue -> MMA: dpre staged (TMEM hi / lo + shared [px][j])
-  unsigned long long* bc_done = bars + 15;    // MMA (b), (c) done: the shared dpre buffer is free
+  unsigned long long* b_done = bars + 15;     // MMA (b) done: the shared dpre buffer is free, the dh accumulator full
+  unsigned long long* c_done = bars + 16;     // MMA (c) of the CTA's last tile done: gW1 | gb1 complete (one phase)
   unsigned* tmem_slot = reinterpret_cast<unsigned*>(bars + BT_NBARS);
 
   // the shuffle makes the warp index provably warp-uniform: role branches are then non-divergent for the
@@ -125,7 +126,8 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
       mbar_init(d1_full + s, 1);
     }
     mbar_init(a23_ready, BT_EPI_WARPS);
-    mbar_init(bc_done, 1);
+    mbar_init(b_done, 1);
+    mbar_init(c_done, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == BT_MMA_WARP) tmem_alloc(tmem_slot, TM_COLS);
@@ -200,6 +202,8 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
             tc_mma_tf32_elect(tmem_base + TM_D2 + (unsigned)(s * 32), (pass == 0 ? d_a2_l : d_a2_h) + (unsigned long long)(ks * (2 * A2_LBO >> 4)),
                               (pass == 1 ? d_b2_l : d_b2_h) + (unsigned long long)(ks * (256 >> 4)), idesc_b,
                               single ? (unsigned)(ks != 0) : (unsigned)((pass | ks) != 0));
+      // (b) alone reads the shared dpre buffer and writes the dh accumulator: the epilogue need not wait for (c)
+      tc_commit_elect(b_done);
       const unsigned long long so = (unsigned long long)(s * (B3_BYTES >> 4));
       const unsigned at = tmem_base + TM_D1 + (unsigned)s * 128u;       // dpre^T hi at +0, lo at +64
 #pragma unroll
@@ -210,8 +214,8 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
             tc_mma_tf32_ts_elect(tmem_base + TM_D3, at + (unsigned)((pass == 0 ? 64 : 0) + ks * 8),
                                  (pass == 1 ? d_b3_l : d_b3_h) + so + (unsigned long long)(ks * (2 * B3_LBO >> 4)), idesc_c,
                                  (single ? (unsigned)(ks != 0) : (unsigned)((pass | ks) != 0)) | (unsigned)(it > 0));
-      tc_commit_elect(bc_done);
       tc_commit_elect(d2_full + s);
+      if (it == ntl - 1) tc_commit_elect(c_done);
       TRACE(2);
     };
     issue_a(0);
@@ -223,11 +227,12 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
     // ---- epilogue: thread = hidden unit j (TMEM lane), 16 pixels (columns) of the tile ----------------
     const int quad = warp & 3, colq = warp >> 2;
     const int j = quad * 32 + lane;
-    float w2r[VP], aw2[VP];
+    float w2r[VP];
+    float2 aw2[VP];                                      // gW2[v][j] over the even / odd pixels of each pair
 #pragma unroll
     for (int v = 0; v < VP; ++v) {
       w2r[v] = (v < V) ? __ldg(W2 + (size_t)v * BT_HID + j) : 0.f;
-      aw2[v] = 0.f;
+      aw2[v] = f32x2(0.f);
     }
     const int a2off = (2 * colq) * A2_SBO + (j >> 2) * A2_LBO + (j & 3) * 4;
     // dh tile of tile `t` (accumulator slot t & 1): D2 row i lives in lane 32 (i / 16) + i % 16, so the drain
@@ -275,25 +280,25 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
       float pre[16];
       tmem_ld16(tq, pre);
       float hi[16], lo[16];
-      const float4* __restrict__ gq = gt + (s * BT_PX + 16 * colq) * 2;
+      const float4* __restrict__ gq = gt + (s * BT_PX + 16 * colq) * (BT_GV / 4);
+      // pixel pairs on the packed f32x2 pipe; the dout tile holds (pixel p, pixel p+1) pairs per variable
 #pragma unroll
-      for (int p = 0; p < 16; ++p) {
-        float gl, gp;
-        gelu_fast_both(pre[p], gl, gp);
-        const float4 go = gq[2 * p];                    // dout * std of this pixel (warp-wide broadcast)
-        float da = w2r[0] * go.x;
-        aw2[0] = fmaf(gl, go.x, aw2[0]);
-        if (VP > 1) { da = fmaf(w2r[1], go.y, da); aw2[1] = fmaf(gl, go.y, aw2[1]); }
-        if (VP > 2) { da = fmaf(w2r[2], go.z, da); aw2[2] = fmaf(gl, go.z, aw2[2]); }
-        if (VP > 3) { da = fmaf(w2r[3], go.w, da); aw2[3] = fmaf(gl, go.w, aw2[3]); }
-        if (VP > 4) {
-          const float4 g2 = gq[2 * p + 1];
-          da = fmaf(w2r[4], g2.x, da); aw2[4] = fmaf(gl, g2.x, aw2[4]);
-          if (VP > 5) { da = fmaf(w2r[5], g2.y, da); aw2[5] = fmaf(gl, g2.y, aw2[5]); }
-          if (VP > 6) { da = fmaf(w2r[6], g2.z, da); aw2[6] = fmaf(gl, g2.z, aw2[6]); }
-          if (VP > 7) { da = fmaf(w2r[7], g2.w, da); aw2[7] = fmaf(gl, g2.w, aw2[7]); }
+      for (int p = 0; p < 16; p += 2) {
+        float2 gl, gp;
+        gelu_fast_both2(make_float2(pre[p], pre[p + 1]), gl, gp);
+        float2 da;
+#pragma unroll
+        for (int q = 0; q < VP / 2; ++q) {
+          const float4 go = gq[(p / 2) * (BT_GV / 2) + q];   // variables 2q, 2q+1 of both pixels (warp-wide broadcast)
+          const float2 g0 = make_float2(go.x, go.y), g1 = make_float2(go.z, go.w);
+          da = q == 0 ? __fmul2_rn(f32x2(w2r[0]), g0) : __ffma2_rn(f32x2(w2r[2 * q]), g0, da);
+          da = __ffma2_rn(f32x2(w2r[2 * q + 1]), g1, da);
+          aw2[2 * q] = __ffma2_rn(gl, g0, aw2[2 * q]);
+          aw2[2 * q + 1] = __ffma2_rn(gl, g1, aw2[2 * q + 1]);
         }
-        split_rm(da * gp, hi[p], lo[p], sp_rnd, sp_msk);
+        const float2 dp = __fmul2_rn(da, gp);
+        split_rm(dp.x, hi[p], lo[p], sp_rnd, sp_msk);
+        split_rm(dp.y, hi[p + 1], lo[p + 1], sp_rnd, sp_msk);
       }
       // dpre^T for (c) goes back into tensor memory, over the pre^T values this thread just read
       tmem_st16(tq, hi);
@@ -302,7 +307,7 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
       if (lane == 0) mbar_arrive(g_free + s);
       if (warp == 0) TRACE(9);
       // the shared dpre buffer was last read by the (b) MMAs of the previous tile
-      mbar_wait(bc_done, ((unsigned)it & 1u) ^ 1u);
+      mbar_wait(b_done, ((unsigned)it & 1u) ^ 1u);
       if (warp == 0) TRACE(10);
 #pragma unroll
       for (int p = 0; p < 16; ++p) {
@@ -316,18 +321,19 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
       __syncwarp();
       if (lane == 0) mbar_arrive(a23_ready);
       if (warp == 0) TRACE(11);
-      // (b), (c) of tile it-1 are done (bc_done above): its dh accumulator is complete
+      // (b) of tile it-1 is done (b_done above): its dh accumulator is complete
       if (it > 0 && colq == ((it - 1) & 3)) drain_dh(it - 1);
     }
     if (colq == ((ntl - 1) & 3)) {
-      mbar_wait(bc_done, (unsigned)(ntl - 1) & 1u);
+      mbar_wait(b_done, (unsigned)(ntl - 1) & 1u);
       drain_dh(ntl - 1);
     }
     // partial records: gW2 share of this pixel quarter; the gW1 | gb1 accumulator (quarter 0 warps)
 #pragma unroll
-    for (int v = 0; v < BT_GV; ++v) myrec[REC_W2 + (colq * BT_GV + v) * BT_HID + j] = (v < VP) ? aw2[v < VP ? v : 0] : 0.f;
+    for (int v = 0; v < BT_GV; ++v)
+      myrec[REC_W2 + (colq * BT_GV + v) * BT_HID + j] = (v < VP) ? aw2[v < VP ? v : 0].x + aw2[v < VP ? v : 0].y : 0.f;
     if (colq == 0) {
-      mbar_wait(bc_done, (unsigned)(ntl - 1) & 1u);
+      mbar_wait(c_done, 0u);
       tc_fence_after();
       float acc[32];
       tmem_ld32(tmem_base + ((unsigned)(quad * 32) << 16) + TM_D3, acc);
@@ -422,8 +428,16 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
           go[v] = (r.valid && v < V) ? r.go[v] * r.sd[v] : 0.f;
           gb2[v] += go[v];
         }
-        gt[(s * BT_PX + px) * 2] = make_float4(go[0], go[1], go[2], go[3]);
-        if (GV > 4) gt[(s * BT_PX + px) * 2 + 1] = make_float4(go[GV - 4], go[GV - 3], go[GV - 2], go[GV - 1]);
+        // pixel-pair layout [pair][variable][pixel of the pair]: the even lane of a pair stores variables 4r, 4r+1, the
+        // odd lane 4r+2, 4r+3, each after one exchange with its partner
+        const bool odd = px & 1;
+#pragma unroll
+        for (int r = 0; r < GV / 4; ++r) {
+          const float a = __shfl_xor_sync(0xffffffffu, odd ? go[4 * r] : go[4 * r + 2], 1);
+          const float c = __shfl_xor_sync(0xffffffffu, odd ? go[4 * r + 1] : go[4 * r + 3], 1);
+          gt[(s * BT_PX + px - odd) * (BT_GV / 4) + 2 * r + odd] = odd ? make_float4(a, go[4 * r + 2], c, go[4 * r + 3])
+                                                               : make_float4(go[4 * r], a, go[4 * r + 1], c);
+        }
       }
       fence_proxy_async();
       __syncwarp();
