@@ -1,5 +1,5 @@
 // extern "C" surface of libfno_sm100.so (include/fno_sm100.h): plan management, argument
-// validation, error reporting.  No torch types, no C++ exceptions across the boundary.
+// validation, error reporting, tensor-map encoding.  No torch types, no C++ exceptions across the boundary.
 #include <cmath>
 #include <cstring>
 #include <mutex>
@@ -31,6 +31,41 @@ int check_launch(const char* what) {
   if (e == cudaSuccess) return FNO_OK;
   set_error("%s: %s", what, cudaGetErrorString(e));
   return FNO_E_CUDA;
+}
+
+namespace {
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn encode_tiled_fn() {
+  static EncodeTiledFn fn = [] {
+    void* f = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess ||
+        q != cudaDriverEntryPointSuccess) {
+      cudaGetLastError();
+      f = nullptr;
+    }
+    return reinterpret_cast<EncodeTiledFn>(f);
+  }();
+  return fn;
+}
+}  // namespace
+
+bool tensor_maps_available() { return encode_tiled_fn() != nullptr; }
+
+bool make_plane_map(CUtensorMap* m, const float* base, unsigned long long pixels, unsigned long long planes,
+                    unsigned box_pixels, unsigned box_planes, unsigned elem_bytes, CUtensorMapL2promotion l2) {
+  const EncodeTiledFn fn = encode_tiled_fn();
+  const unsigned per = elem_bytes / 4;   // floats per element
+  if (fn == nullptr || base == nullptr || (per != 1 && per != 2) || pixels % per != 0 || box_pixels % per != 0) return false;
+  const cuuint64_t gdim[2] = {pixels / per, planes};
+  const cuuint64_t gstr[1] = {pixels * 4ull};
+  const cuuint32_t box[2] = {box_pixels / per, box_planes};
+  const cuuint32_t estr[2] = {1, 1};
+  return fn(m, per == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), gdim,
+            gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, l2,
+            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 namespace {

@@ -1,5 +1,6 @@
 // Shared declarations for libfno_sm100.so (B200 / sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 
 #include <atomic>
@@ -85,11 +86,40 @@ bool mix_tc_supported(const Plan* p, int Ci, int Co);
 bool pointwise_tc_supported(int Cin, int Cout);
 int launch_wgrad_tc_rows128(const float* ds, const float* a, float* part, int B, int Co, int Ci, long N, int max_parts,
                             int* nparts, cudaStream_t st);
-int launch_wgrad_reduce(const float* part, float* gW, float* gb, int nparts, int Co, int Ci, cudaStream_t st);
 int launch_wgrad_tc(const float* ds, const float* a, float* part, int B, int Co, int Ci, long N, int max_parts, int* nparts,
                     cudaStream_t st);
 int launch_pointwise_tc(const float* in, const float* W, const float* bias, float* out, int B, int Co, int Ci, long N,
                         int transpose, cudaStream_t st);
+
+// ---- split-K reduction ------------------------------------------------------------------------
+// The weight gradients are computed split-K: every CTA writes a record of partial sums and one more launch sums the
+// records in a fixed order, so the result is deterministic.  Output k of a segment reads record offset
+//   col + k                                    (row == 0: a contiguous run), or
+//   (k / row) * stride + col + k % row         (row > 0: a [n / row][row] matrix stored with pitch `stride`),
+// plus q * copy_stride for each of the `copies` sub-records of one record that sum into the same output.
+// A null dst skips the segment's stores; unused segments have n == 0.
+struct ReduceSeg {
+  float* dst = nullptr;
+  int n = 0;
+  int col = 0;
+  int row = 0;
+  int stride = 0;
+  int copies = 1;
+  int copy_stride = 0;
+};
+struct ReduceSegs {
+  ReduceSeg s[4];
+};
+// out = sum over the nparts records of length reclen at `part`; one warp per output element.
+int launch_partial_reduce(const float* part, int nparts, int reclen, const ReduceSegs& segs, cudaStream_t st);
+
+// ---- 2-D tensor maps (cuTensorMapEncodeTiled, resolved once through the runtime: no link-time libcuda dependency) -----
+bool tensor_maps_available();
+// The [planes][pixels] view of a channel-first f32 tensor with a box of {box_pixels, box_planes}, zero fill outside.
+// elem_bytes 4 reads a row as FLOAT32; 8 as UINT64 float pairs (pixels and box_pixels even), which fits twice the
+// pixels into the 256-element box limit.  False when the entry point is missing or the encoding is rejected.
+bool make_plane_map(CUtensorMap* m, const float* base, unsigned long long pixels, unsigned long long planes,
+                    unsigned box_pixels, unsigned box_planes, unsigned elem_bytes, CUtensorMapL2promotion l2);
 
 // ---- device helpers --------------------------------------------------------------------------
 // exact unsigned 32-bit division by a run-time constant (Granlund-Montgomery): 4 instructions instead
@@ -259,6 +289,13 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned by
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
                    smem_u32(dst)),
                "l"(src), "r"(bytes), "r"(smem_u32(bar))
+               : "memory");
+}
+// one box of a 2-D tensor map at element coordinates {c0, c1}; completes on `bar` with the box's full byte count
+// (elements outside the tensor are zero-filled and still counted)
+__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, unsigned long long* bar) {
+  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
+               ::"r"(smem_u32(dst)), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
                : "memory");
 }
 

@@ -502,32 +502,6 @@ head_bwd_tc_kernel(const float* __restrict__ h, const float* __restrict__ dout, 
   if (warp == BT_MMA_WARP) tmem_dealloc(tmem_base, TM_COLS);
 }
 
-// gW1 [128][C], gb1 [128], gW2 [V][128], gb2 [V] from the per-CTA records; one warp per output element,
-// fixed summation order (deterministic)
-__global__ void __launch_bounds__(128)
-head_bwd_tc_reduce_kernel(const float* __restrict__ rec, int nrec, float* __restrict__ gW1, float* __restrict__ gb1,
-                          float* __restrict__ gW2, float* __restrict__ gb2, int C, int V) {
-  const int idx = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  const int n1 = BT_HID * C, n2 = n1 + BT_HID, n3 = n2 + V * BT_HID, n4 = n3 + V;
-  if (idx >= n4) return;
-  int base, inner, istride;
-  float* dst;
-  if (idx < n1) { const int j = idx / C, c = idx - j * C; base = REC_W1 + j * BT_NC + c; inner = 1; istride = 0; dst = gW1 + idx; }
-  else if (idx < n2) { const int j = idx - n1; base = REC_W1 + j * BT_NC + C; inner = 1; istride = 0; dst = gb1 + j; }
-  else if (idx < n3) { const int k = idx - n2, v = k / BT_HID, j = k - v * BT_HID; base = REC_W2 + v * BT_HID + j; inner = 4; istride = BT_GV * BT_HID; dst = gW2 + k; }
-  else { const int v = idx - n3; base = REC_B2 + v; inner = 2; istride = BT_GV; dst = gb2 + v; }
-  float s = 0.f;
-  const int total = nrec * inner;
-  for (int t = lane; t < total; t += 32) {
-    const int r = t / inner, q = t - r * inner;
-    s += rec[(size_t)r * REC_LEN + base + q * istride];
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (lane == 0) *dst = s;
-}
-
 }  // namespace
 
 size_t head_bwd_tc_workspace_bytes() { return sizeof(float) * (size_t)148 * REC_LEN; }
@@ -588,8 +562,11 @@ extern "C" int fno_head_bwd_tc(const float* h, const float* dout, const float* W
   count_launch();
   rc = check_launch("head_bwd_tc_kernel");
   if (rc != FNO_OK) return rc;
-  const int nout = BT_HID * C + BT_HID + V * BT_HID + V;
-  head_bwd_tc_reduce_kernel<<<(nout * 32 + 127) / 128, 128, 0, st>>>(rec, ctas, gW1, gb1, gW2, gb2, C, V);
-  count_launch();
-  return check_launch("head_bwd_tc_reduce_kernel");
+  // gW1 [128][C], gb1 [128] (column C of the gW1 rows), gW2 [V][128] summed over 4 copies, gb2 [V] over 2
+  ReduceSegs segs;
+  segs.s[0] = {gW1, BT_HID * C, REC_W1, C, BT_NC};
+  segs.s[1] = {gb1, BT_HID, REC_W1 + C, 1, BT_NC};
+  segs.s[2] = {gW2, V * BT_HID, REC_W2, 0, 0, 4, BT_GV * BT_HID};
+  segs.s[3] = {gb2, V, REC_B2, 0, 0, 2, BT_GV};
+  return launch_partial_reduce(rec, ctas, REC_LEN, segs, st);
 }

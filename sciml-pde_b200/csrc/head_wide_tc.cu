@@ -291,21 +291,6 @@ head_bwd_wide_kernel(const float* __restrict__ h, const float* __restrict__ dout
   if (warp == HW_EPI_WARPS) tmem_dealloc(tmem_base, HW_TM_COLS);
 }
 
-// gW2 [V][128], gb2 [V] from the per-CTA records: one warp per output element, fixed order
-__global__ void __launch_bounds__(128)
-head_wide_reduce_kernel(const float* __restrict__ rec, int nrec, float* __restrict__ gW2, float* __restrict__ gb2, int V) {
-  const int idx = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  const int n1 = V * HW_HID;
-  if (idx >= n1 + V) return;
-  const int src = idx < n1 ? idx : HW_VP * HW_HID + (idx - n1);
-  float s = 0.f;
-  for (int t = lane; t < nrec; t += 32) s += rec[(size_t)t * HW_REC + src];
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (lane == 0) (idx < n1 ? gW2[idx] : gb2[idx - n1]) = s;
-}
-
 constexpr int HW_WG_PARTS = 148;
 
 // ------------------------------------------------------------------------------------------
@@ -539,15 +524,19 @@ extern "C" int fno_head_bwd_wide_tc(const float* h, const float* dout, const flo
   count_launch();
   int rc = check_launch("head_bwd_wide_kernel");
   if (rc != FNO_OK) return rc;
-  head_wide_reduce_kernel<<<((V * HW_HID + V) * 32 + 127) / 128, 128, 0, st>>>(rec, ctas, gW2, gb2, V);
-  count_launch();
-  rc = check_launch("head_wide_reduce_kernel");
+  ReduceSegs segs2;                              // gW2 [V][128] | gb2 [V]
+  segs2.s[0] = {gW2, V * HW_HID, 0};
+  segs2.s[1] = {gb2, V, HW_VP * HW_HID};
+  rc = launch_partial_reduce(rec, ctas, HW_REC, segs2, st);
   if (rc != FNO_OK) return rc;
   // gW1 [128][C] | gb1 [128] = sum over all positions of dpre (x) [h ; 1]  (dpre is zero in the padding)
   int nparts = 0;
   rc = launch_wgrad_tc_rows128(dpre, h, part, B, HW_HID, C, g.plane, HW_WG_PARTS, &nparts, st);
   if (rc != FNO_OK) return rc;
-  return launch_wgrad_reduce(part, gW1, gb1, nparts, HW_HID, C, st);
+  ReduceSegs segs1;                              // records [nparts][128][C + 1]
+  segs1.s[0] = {gW1, HW_HID * C, 0, C, C + 1};
+  segs1.s[1] = {gb1, HW_HID, C, 1, C + 1};
+  return launch_partial_reduce(part, nparts, HW_HID * (C + 1), segs1, st);
 }
 
 extern "C" int fno_head_fwd_wide_tc(const float* h, const float* W1, const float* b1, const float* W2, const float* b2,

@@ -573,38 +573,37 @@ lift_bwd2_kernel(const float* __restrict__ x, const float* __restrict__ grid, co
   }
 }
 
-// out[i] = sum over partials in fixed order (deterministic); one warp per output element.
-// Output i of each partial record is routed to dst0 (i < n0), dst1 (i < n0 + n1), ... by `segs`.
-struct ReduceSegs {
-  float* dst[4];
-  int n[4];          // element counts (sum = record length)
-  int row[4];        // 0: contiguous copy; >0: the segment is a [rows][row] matrix taken from a record
-  int stride[4];     // laid out [rows][stride] starting at column `col`
-  int col[4];
-};
-
+// The split-K reduction of every weight gradient (common.cuh): output k of segment s, one warp per output.  Lanes stride
+// the records (and, with copies > 1, the copies of one record: t = record * copies + copy), then a fixed xor tree.
 __global__ void __launch_bounds__(128)
 partial_reduce_kernel(const float* __restrict__ part, int nparts, int reclen, ReduceSegs segs) {
-  const int idx = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  int k = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  int total = 0;
+  // unrolled, so that every segment is read from the parameter bank (a run-time index would copy segs to the stack)
+  ReduceSeg g = segs.s[0];
 #pragma unroll
-  for (int s = 0; s < 4; ++s) total += segs.n[s];
-  if (idx >= total) return;
-  int s = 0, k = idx;
-  while (s < 3 && k >= segs.n[s]) { k -= segs.n[s]; ++s; }
+  for (int s = 1; s < 4; ++s)
+    if (k >= g.n) { k -= g.n; g = segs.s[s]; }
+  if (k >= g.n) return;
   int src;
-  if (segs.row[s] > 0) {
-    const int r = k / segs.row[s], c = k - r * segs.row[s];
-    src = r * segs.stride[s] + segs.col[s] + c;
+  if (g.row > 0) {
+    const int r = k / g.row, c = k - r * g.row;
+    src = r * g.stride + g.col + c;
   } else {
-    src = segs.col[s] + k;
+    src = g.col + k;
   }
   float sum = 0.f;
-  for (int p = lane; p < nparts; p += 32) sum += part[(size_t)p * reclen + src];
+  if (g.copies == 1) {
+    for (int p = lane; p < nparts; p += 32) sum += part[(size_t)p * reclen + src];
+  } else {
+    for (int t = lane; t < nparts * g.copies; t += 32) {
+      const int r = t / g.copies, q = t - r * g.copies;
+      sum += part[(size_t)r * reclen + src + q * g.copy_stride];
+    }
+  }
 #pragma unroll
   for (int off = 16; off > 0; off >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, off);
-  if (lane == 0 && segs.dst[s] != nullptr) segs.dst[s][k] = sum;
+  if (lane == 0 && g.dst != nullptr) g.dst[k] = sum;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -961,14 +960,11 @@ int launch_head_bwd(const float* h, const float* dout, const float* W1, const fl
   if (rc != FNO_OK) return rc;
   const int reclen = HID * CP + HID + VP * HID + VP;
   ReduceSegs segs;
-  segs.dst[0] = gW1; segs.n[0] = HID * C; segs.row[0] = C; segs.stride[0] = CP; segs.col[0] = 0;
-  segs.dst[1] = gb1; segs.n[1] = HID;     segs.row[1] = 0; segs.stride[1] = 0;  segs.col[1] = HID * CP;
-  segs.dst[2] = gW2; segs.n[2] = V * HID; segs.row[2] = 0; segs.stride[2] = 0;  segs.col[2] = HID * CP + HID;
-  segs.dst[3] = gb2; segs.n[3] = V;       segs.row[3] = 0; segs.stride[3] = 0;  segs.col[3] = HID * CP + HID + VP * HID;
-  const int total_out = HID * C + HID + V * HID + V;
-  partial_reduce_kernel<<<(total_out * 32 + 127) / 128, 128, 0, st>>>(part, ctas, reclen, segs);
-  count_launch();
-  return check_launch("partial_reduce_kernel(head)");
+  segs.s[0] = {gW1, HID * C, 0, C, CP};
+  segs.s[1] = {gb1, HID, HID * CP};
+  segs.s[2] = {gW2, V * HID, HID * CP + HID};
+  segs.s[3] = {gb2, V, HID * CP + HID + VP * HID};
+  return launch_partial_reduce(part, ctas, reclen, segs, st);
 }
 
 int pick_cp(int C) {
@@ -993,6 +989,13 @@ int launch_pad_zero(float* h, const PixGeo& g, long planes, cudaStream_t st) {
 }  // namespace fno
 
 namespace fno {
+int launch_partial_reduce(const float* part, int nparts, int reclen, const ReduceSegs& segs, cudaStream_t st) {
+  const int total = segs.s[0].n + segs.s[1].n + segs.s[2].n + segs.s[3].n;
+  partial_reduce_kernel<<<(total * 32 + 127) / 128, 128, 0, st>>>(part, nparts, reclen, segs);
+  count_launch();
+  return check_launch("partial_reduce_kernel");
+}
+
 // zero padding of a trunk-layout gradient tensor (used by head_bwd_tc.cu as well)
 int head_pad_zero(float* dh, int R_in, int W_in, int R_out, int Wp, long planes, cudaStream_t st) {
   return launch_pad_zero(dh, make_geo(R_in, W_in, R_out, Wp), planes, st);
@@ -1126,13 +1129,9 @@ extern "C" int fno_lift_bwd(const float* x, const float* grid, const float* stat
         int rc2 = check_launch("lift_bwd2_kernel");
         if (rc2 != FNO_OK) return rc2;
         ReduceSegs segs2;
-        for (int s = 0; s < 4; ++s) { segs2.dst[s] = nullptr; segs2.n[s] = 0; segs2.row[s] = 0; segs2.stride[s] = 0; segs2.col[s] = 0; }
-        segs2.dst[0] = gW0; segs2.n[0] = C * F; segs2.row[0] = F; segs2.stride[0] = F + 1; segs2.col[0] = 0;
-        segs2.dst[1] = gb0; segs2.n[1] = C;     segs2.row[1] = 1; segs2.stride[1] = F + 1; segs2.col[1] = F;
-        const int total_out2 = C * F + C;
-        partial_reduce_kernel<<<(total_out2 * 32 + 127) / 128, 128, 0, st>>>(part0, ctas, C * (F + 1), segs2);
-        count_launch();
-        return check_launch("partial_reduce_kernel(lift)");
+        segs2.s[0] = {gW0, C * F, 0, F, F + 1};
+        segs2.s[1] = {gb0, C, F, 1, F + 1};
+        return launch_partial_reduce(part0, ctas, C * (F + 1), segs2, st);
       }
     }
   }
@@ -1154,13 +1153,9 @@ extern "C" int fno_lift_bwd(const float* x, const float* grid, const float* stat
   int rc = check_launch("lift_bwd_kernel");
   if (rc != FNO_OK) return rc;
   ReduceSegs segs;
-  for (int s = 0; s < 4; ++s) { segs.dst[s] = nullptr; segs.n[s] = 0; segs.row[s] = 0; segs.stride[s] = 0; segs.col[s] = 0; }
-  segs.dst[0] = gW0; segs.n[0] = C * F; segs.row[0] = F; segs.stride[0] = F + 1; segs.col[0] = 0;
-  segs.dst[1] = gb0; segs.n[1] = C;     segs.row[1] = 1; segs.stride[1] = F + 1; segs.col[1] = F;
-  const int total_out = C * F + C;
-  partial_reduce_kernel<<<(total_out * 32 + 127) / 128, 128, 0, st>>>(part, ctas * KSPL, C * (F + 1), segs);
-  count_launch();
-  return check_launch("partial_reduce_kernel(lift)");
+  segs.s[0] = {gW0, C * F, 0, F, F + 1};
+  segs.s[1] = {gb0, C, F, 1, F + 1};
+  return launch_partial_reduce(part, ctas * KSPL, C * (F + 1), segs, st);
 }
 
 extern "C" int fno_head_fwd(const float* h, const float* W1, const float* b1, const float* W2, const float* b2,

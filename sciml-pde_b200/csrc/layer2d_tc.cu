@@ -31,8 +31,6 @@
 //   MMA warp         18 tcgen05.mma per row into a double-buffered accumulator         ready -> mma_done
 //   8 epilogue warps tcgen05.ld, GELU, stores                                          mma_done -> ready
 // (`ready[s]` collects the A buffer, the T2 operand tile and the free accumulator of a row: one wait in the MMA warp)
-#include <cuda.h>
-
 #include <cstdlib>
 #include <cstring>
 
@@ -57,13 +55,9 @@ constexpr int L2_NR = 4;          // T2 tiles in flight (bulk copies into a shar
 constexpr int L2_NS = 6;          // activation rows in flight with the tensor-map path (3 per row parity)
 constexpr int L2_PD = 3;          // own rows of activation copies in flight per converter warp (= 6 rows ahead)
 
-// 2-D tiled TMA: box {Wm pixels, C planes} of the [planes][pixels] view of an activation tensor <-> dense [C][Wm] shared memory.
-// The tensor map takes element coordinates, so the 8-byte-aligned rows of the 130-wide planes need no special casing.
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-               ::"r"(smem_u32(dst)), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-               : "memory");
-}
+// 2-D tiled TMA: box {Wm pixels, C planes} of the [planes][pixels] view of an activation tensor <-> dense [C][Wm] shared memory
+// (loads through tma_load_2d).  The tensor map takes element coordinates, so the 8-byte-aligned rows of the 130-wide planes need
+// no special casing.
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, int c0, int c1, const void* src) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];"
                ::"l"(map), "r"(c0), "r"(c1), "r"(smem_u32(src))
@@ -759,35 +753,6 @@ size_t layer2d_smem_bytes(int KQ, int C, int Wm, bool tma) {
                           (size_t)L2_NR * ((C + 7) / 8) * KQ * 8 + staging) + 128 + 16 + (9 + 2 * L2_NR + 8 * L2_PD) * 8 + 16;
 }
 
-// ---- tensor maps (driver entry point resolved through the runtime: no link-time dependency on libcuda) ----------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_tiled_fn() {
-  static EncodeTiledFn fn = [] {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess) {
-      cudaGetLastError();
-      f = nullptr;
-    }
-    return reinterpret_cast<EncodeTiledFn>(f);
-  }();
-  return fn;
-}
-// [planes][pixels] f32 view of an activation tensor, box {Wm pixels, C planes}
-bool make_act_map(CUtensorMap* m, const float* base, unsigned long long pixels, unsigned long long planes, unsigned Wm, unsigned C) {
-  EncodeTiledFn fn = encode_tiled_fn();
-  if (fn == nullptr || base == nullptr) return false;
-  const cuuint64_t gdim[2] = {pixels, planes};
-  const cuuint64_t gstr[1] = {pixels * 4ull};
-  const cuuint32_t box[2] = {Wm, C};
-  const cuuint32_t estr[2] = {1, 1};
-  return fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 template <int KA, int NPAD, int CWQ, int CX, bool GELU, bool SOUT, bool TMA>
 int launch_layer2d_k(const L2Args& args, cudaStream_t st, bool attr_only) {
   using Cfg = L2Cfg<KA, NPAD, CWQ>;
@@ -804,8 +769,10 @@ int launch_layer2d_k(const L2Args& args, cudaStream_t st, bool attr_only) {
   memset(&ma, 0, sizeof(ma)); memset(&mo, 0, sizeof(mo)); memset(&ms, 0, sizeof(ms));
   if (TMA) {
     const unsigned long long pixels = (unsigned long long)args.RS * args.W, planes = (unsigned long long)(args.total_tiles / args.RS) * args.C;
-    if (!make_act_map(&ma, args.a, pixels, planes, 32, args.C) || !make_act_map(&mo, args.out, pixels, planes, Wm, args.C) ||
-        (SOUT && !make_act_map(&ms, args.s_out, pixels, planes, Wm, args.C))) {
+    const auto l2 = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
+    if (!make_plane_map(&ma, args.a, pixels, planes, 32, args.C, 4, l2) ||
+        !make_plane_map(&mo, args.out, pixels, planes, Wm, args.C, 4, l2) ||
+        (SOUT && !make_plane_map(&ms, args.s_out, pixels, planes, Wm, args.C, 4, l2))) {
       set_error("layer2d_tc: cuTensorMapEncodeTiled failed");
       return FNO_E_CUDA;
     }
@@ -819,7 +786,7 @@ int launch_layer2d_k(const L2Args& args, cudaStream_t st, bool attr_only) {
 // tensor-map eligibility: 16-byte aligned tensors and plane pitch, box rows a multiple of 16 bytes
 bool layer2d_tma_ok(const L2Args& a) {
   static const bool off = [] { const char* e = std::getenv("FNO_LAYER_TMA"); return e != nullptr && e[0] == '0'; }();
-  if (off || encode_tiled_fn() == nullptr) return false;
+  if (off || !tensor_maps_available()) return false;
   const int Wm = a.W < 128 ? a.W : 128;
   if (((long)a.RS * a.W) % 4 != 0 || Wm % 4 != 0 || (long)a.RS * a.W >= (1L << 31)) return false;
   // every row's column window must start 16-byte aligned: W % 4 == 0, or W = 130 (window [2, 130) on odd rows)

@@ -9,9 +9,6 @@
 //     huge K = B*N and a tiny output, so it is a split-K reduction: a CTA stages a K-slab of both
 //     operands in shared memory, each warp owns a T x T output tile with lanes striding K, and
 //     per-CTA partials are combined by a second fixed-order pass (deterministic, no atomics).
-#include <cuda.h>
-
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -293,83 +290,40 @@ wgrad_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a, 
 }
 
 // ------------------------------------------------------------------------------------------
-// v2 of the weight gradient: TMA-fed (cp.async.bulk, 1-D) slabs with an mbarrier full/empty ring.
-// Warp 0 streams slab after slab -- one bulk copy of KT pixels per channel row of ds and
-// of a -- into a WG2_STAGES-deep ring; the warps each own one T x T output tile with lanes
-// over pixel quads (LDS.128: 2T loads per 4 T^2 FMA).  Nothing but the bulk copies touches global
-// memory in the steady state, so the kernel streams at the HBM rate set by its 8 bytes/pixel/channel.
+// v2 of the weight gradient: TMA-fed slabs with an mbarrier full/empty ring.  Warp 0 streams slab after slab into a
+// WG2_STAGES-deep ring; the warps each own one T x T output tile with lanes over pixel quads (LDS.128: 2T loads per
+// 4 T^2 FMA).  Nothing but the tensor-map copies touches global memory in the steady state, so the kernel streams at the
+// HBM rate set by its 8 bytes/pixel/channel.
 // ------------------------------------------------------------------------------------------
 constexpr int WG2_STAGES = 2;
-constexpr int WG2_KT = 512;      // pixels per slab: 2 KB per bulk copy (the TMA unit retires ~1 copy / 46 cycles / SM,
-                                 // so 512-byte copies cap the stream at ~3 TB/s -- profiles/r1_d)
+constexpr int WG2_KT = 512;      // pixels per slab: the 256-element box limit, in float pairs
 constexpr int WG2_MAXW = 8;      // consumer warps per CTA
-// TMAP: a slab is TWO 2-D tensor-map copies -- box {512 pixels, C planes} of the [planes][pixels] view of ds and of a, with
-// the row taken as 8-byte elements (PAIRS) so that 512 pixels fit the 256-element box limit: 40 KB per copy at width 20
-// instead of Co + Ci bulk copies of 2 KB.  Pixels past the end of a sample are zero-filled by the TMA unit (and still counted by
-// complete_tx).  Measured at cfg 1 (B = 128, profiles/r2g_wgrad_forms.md): bulk copies 124 us, the same ring fed by tensor
+// A slab is TWO 2-D tensor-map copies -- box {512 pixels, C planes} of the [planes][pixels] view of ds and of a, with the row
+// taken as 8-byte elements so that 512 pixels fit the 256-element box limit: 40 KB per copy at width 20 instead of Co + Ci
+// bulk copies of 2 KB.  Pixels past the end of a sample are zero-filled by the TMA unit (and still counted by complete_tx).
+// Measured at cfg 1 (B = 128, profiles/r2g_wgrad_forms.md): one bulk copy per channel row 124 us, the same ring fed by tensor
 // maps 93 us, + FULL 89 us; a kernel that only waits for its slabs 79-85 us in every form (the TMA feed tops out at ~4.5 TB/s),
-// and every bulk copy costs ~40 ns of issue on top (256-pixel slabs with twice the copies: 171 us).
-__device__ __forceinline__ void wg2_tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-               ::"r"(smem_u32(dst)), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar))
-               : "memory");
-}
-
-// ---- tensor maps of the operand feed (driver entry point resolved through the runtime: no link-time libcuda dependency) ----
-typedef CUresult (*Wg2EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                     const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-Wg2EncodeTiledFn wg2_encode_fn() {
-  static Wg2EncodeTiledFn fn = [] {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess) {
-      cudaGetLastError();
-      f = nullptr;
-    }
-    return reinterpret_cast<Wg2EncodeTiledFn>(f);
-  }();
-  return fn;
-}
-// [planes][pixels] f32 view of a channel-first tensor, box {kt pixels, c planes}, zero fill outside
-bool wg2_make_map(CUtensorMap* m, const float* base, unsigned long long pixels, unsigned long long planes, unsigned kt, unsigned c) {
-  Wg2EncodeTiledFn fn = wg2_encode_fn();
-  if (fn == nullptr || base == nullptr || c == 0 || c > 256 || kt > 512 || (pixels & 1ull)) return false;
-  const cuuint64_t gdim[2] = {pixels / 2, planes};
-  const cuuint64_t gstr[1] = {pixels * 4ull};
-  const cuuint32_t box[2] = {kt / 2, c};
-  const cuuint32_t estr[2] = {1, 1};
-  return fn(m, CU_TENSOR_MAP_DATA_TYPE_UINT64, 2, const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-bool wg2_use_maps() {
-  static const bool on = [] { const char* e = std::getenv("FNO_WG2"); return !(e != nullptr && e[0] == '0'); }();
-  return on && wg2_encode_fn() != nullptr;
-}
+// and every bulk copy costs ~40 ns of issue on top.
 
 // DGRAD: the same pass also produces the bypass data gradient dx[b, i, p] = sum_o W[o, i] ds[b, o, p]
 // (autograd of nn.Conv2d(C, C, 1), fno/fno.py:162) from the ds slab that is already in shared memory --
 // one read of the ds tensor per layer instead of two.  Thread = two adjacent pixels of the 512-pixel slab
 // (8 consumer warps), all Ci outputs in registers, weight rows broadcast with LDS.128.
-template <int T, bool DGRAD, int KT2 = WG2_KT, int NST = WG2_STAGES, bool TMAP = false, bool PAIRS = false, bool FULL = false>
+template <int T, bool DGRAD, bool FULL>
 __global__ void __launch_bounds__(32 * WG2_MAXW)
-wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a, float* __restrict__ part, int Co,
-                      int Ci, long N, int slabs_per_sample, long total_slabs, long slabs_per_cta, int tiles_i,
-                      int ntiles, int nwarps, int KH, const float* __restrict__ Wm, float* __restrict__ dx,
-                      const __grid_constant__ CUtensorMap tm_ds, const __grid_constant__ CUtensorMap tm_a) {
-  static_assert(!DGRAD || KT2 == WG2_KT, "the fused data gradient covers a 512-pixel slab with 256 threads");
-  constexpr bool EARLY_REFILL = NST > 2;
-  extern __shared__ __align__(128) float wg2_sm[];  // NST x ([Co][KT2] ds slab, [Ci][KT2] a slab), then barriers
+wgrad2_partial_kernel(float* __restrict__ part, int Co, int Ci, long N, int slabs_per_sample, long total_slabs,
+                      long slabs_per_cta, int tiles_i, int ntiles, int nwarps, int KH, const float* __restrict__ Wm,
+                      float* __restrict__ dx, const __grid_constant__ CUtensorMap tm_ds, const __grid_constant__ CUtensorMap tm_a) {
+  extern __shared__ __align__(128) float wg2_sm[];  // WG2_STAGES x ([Co][WG2_KT] ds slab, [Ci][WG2_KT] a slab), then barriers
   float* const sm = wg2_sm;
   const int rows = Co + Ci;
-  unsigned long long* full = reinterpret_cast<unsigned long long*>(sm + (size_t)NST * rows * KT2);
-  unsigned long long* empty = full + NST;
-  float* ws = reinterpret_cast<float*>(empty + NST);            // DGRAD: W [Co][2T] (rows zero-padded)
+  unsigned long long* full = reinterpret_cast<unsigned long long*>(sm + (size_t)WG2_STAGES * rows * WG2_KT);
+  unsigned long long* empty = full + WG2_STAGES;
+  float* ws = reinterpret_cast<float*>(empty + WG2_STAGES);            // DGRAD: W [Co][2T] (rows zero-padded)
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   if (threadIdx.x == 0) {
-    for (int s = 0; s < NST; ++s) {
+    for (int s = 0; s < WG2_STAGES; ++s) {
       mbar_init(full + s, 1);
       mbar_init(empty + s, nwarps);
     }
@@ -386,39 +340,28 @@ wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a,
   long s_end = s_begin + slabs_per_cta;
   if (s_end > total_slabs) s_end = total_slabs;
 
-  // ---- producer duty (warp 0): one bulk copy per channel row of ds and of a per slab.  There is no
+  // ---- producer duty (warp 0): one tensor-map copy of ds and one of a per slab.  There is no
   // dedicated producer warp: a ninth warp would put three warps on one SM sub-partition and cap the kernel at
   // 168 registers (16 K registers per sub-partition), which the fused data-gradient phase does not fit.
   auto produce = [&](long slab) {
     if (slab >= s_end) return;
     const int it = (int)(slab - s_begin);
-    const int stage = it % NST;
-    const unsigned ph = (unsigned)(it / NST) & 1u;
+    const int stage = it % WG2_STAGES;
+    const unsigned ph = (unsigned)(it / WG2_STAGES) & 1u;
     mbar_wait(empty + stage, ph ^ 1u);            // every consumer warp is done with the slab that used this stage
     const long b = slab / slabs_per_sample;
-    const long k0 = (slab - b * slabs_per_sample) * KT2;
-    float* dst = sm + (size_t)stage * rows * KT2;
-    if (TMAP) {
-      if (lane == 0) {
-        mbar_arrive_expect_tx(full + stage, (unsigned)(KT2 * sizeof(float)) * (unsigned)rows);   // whole boxes, zero fill included
-        const int c0 = PAIRS ? (int)(k0 >> 1) : (int)k0;
-        wg2_tma_load_2d(dst, &tm_ds, c0, (int)(b * Co), full + stage);
-        wg2_tma_load_2d(dst + (size_t)Co * KT2, &tm_a, c0, (int)(b * Ci), full + stage);
-      }
-      __syncwarp();
-      return;
+    const long k0 = (slab - b * slabs_per_sample) * WG2_KT;
+    float* dst = sm + (size_t)stage * rows * WG2_KT;
+    if (lane == 0) {
+      mbar_arrive_expect_tx(full + stage, (unsigned)(WG2_KT * sizeof(float)) * (unsigned)rows);   // whole boxes, zero fill included
+      const int c0 = (int)(k0 >> 1);                                                           // in float pairs
+      tma_load_2d(dst, &tm_ds, c0, (int)(b * Co), full + stage);
+      tma_load_2d(dst + (size_t)Co * WG2_KT, &tm_a, c0, (int)(b * Ci), full + stage);
     }
-    const long left = N - k0;
-    const unsigned bytes = (unsigned)((left < KT2 ? left : KT2) * sizeof(float));
-    if (lane == 0) mbar_arrive_expect_tx(full + stage, bytes * (unsigned)rows);
     __syncwarp();
-    for (int c = lane; c < rows; c += 32) {
-      const float* src = (c < Co) ? (ds + ((size_t)b * Co + c) * N + k0) : (a + ((size_t)b * Ci + (c - Co)) * N + k0);
-      bulk_g2s(dst + (size_t)c * KT2, src, bytes, full + stage);
-    }
   };
   if (warp == 0) {
-    for (int s = 0; s < NST; ++s) produce(s_begin + s);
+    for (int s = 0; s < WG2_STAGES; ++s) produce(s_begin + s);
   }
 
   // ---- consumer warps: (tile, pixel part) each; a tile is a T x T block of outputs ------------
@@ -431,8 +374,8 @@ wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a,
   // immediates, and the two warps of a tile row share the bias rows (T/2 each) so that all warps carry the same work
   const bool bias_hi = FULL && ti != 0;
   const bool bias_tile = has_tile && (FULL || ti == 0);
-  const float* const ds_t = sm + (size_t)to * KT2 + 4 * lane;
-  const float* const a_t = sm + (size_t)(Co + ti) * KT2 + 4 * lane;
+  const float* const ds_t = sm + (size_t)to * WG2_KT + 4 * lane;
+  const float* const a_t = sm + (size_t)(Co + ti) * WG2_KT + 4 * lane;
   float acc[T][T];
   float accb[T];
 #pragma unroll
@@ -441,28 +384,26 @@ wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a,
 #pragma unroll
     for (int c = 0; c < T; ++c) acc[r][c] = 0.f;
   }
-  const int steps = KT2 / 128;                    // 128 pixels (32 lanes x 4) per step
+  const int steps = WG2_KT / 128;                    // 128 pixels (32 lanes x 4) per step
   for (long slab = s_begin; slab < s_end; ++slab) {
     const int it = (int)(slab - s_begin);
-    const int stage = it % NST;
-    const unsigned ph = (unsigned)(it / NST) & 1u;
-    // deep ring: refill the stage of the PREVIOUS slab now (the other warps left it a whole slab of products ago)
-    if (EARLY_REFILL && warp == 0 && it > 0) produce(slab - 1 + NST);
+    const int stage = it % WG2_STAGES;
+    const unsigned ph = (unsigned)(it / WG2_STAGES) & 1u;
     mbar_wait(full + stage, ph);
     const long b = slab / slabs_per_sample;
-    const long left = N - (slab - b * slabs_per_sample) * KT2;
+    const long left = N - (slab - b * slabs_per_sample) * WG2_KT;
     if (has_tile) {
       for (int st = kh; st < steps; st += KH) {
         const int px = st * 128 + 4 * lane;       // a short slab at the end of a sample ends on a quad (N % 4 == 0)
         if (px >= left) break;
-        const float* ds_s = sm + (size_t)stage * rows * KT2 + px;
-        const float* a_s = ds_s + (size_t)Co * KT2;
-        const int soff = stage * rows * KT2 + st * 128;
+        const float* ds_s = sm + (size_t)stage * rows * WG2_KT + px;
+        const float* a_s = ds_s + (size_t)Co * WG2_KT;
+        const int soff = stage * rows * WG2_KT + st * 128;
         float4 dv[T];
 #pragma unroll
         for (int r = 0; r < T; ++r) {
-          if (FULL) dv[r] = *reinterpret_cast<const float4*>(ds_t + soff + r * KT2);
-          else dv[r] = (to + r < Co) ? *reinterpret_cast<const float4*>(ds_s + (to + r) * KT2) : make_float4(0.f, 0.f, 0.f, 0.f);
+          if (FULL) dv[r] = *reinterpret_cast<const float4*>(ds_t + soff + r * WG2_KT);
+          else dv[r] = (to + r < Co) ? *reinterpret_cast<const float4*>(ds_s + (to + r) * WG2_KT) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
         if (FULL) {
           if (!bias_hi) {
@@ -479,8 +420,8 @@ wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a,
 #pragma unroll
         for (int c = 0; c < T; ++c) {
           float4 av;
-          if (FULL) av = *reinterpret_cast<const float4*>(a_t + soff + c * KT2);
-          else av = (ti + c < Ci) ? *reinterpret_cast<const float4*>(a_s + (ti + c) * KT2) : make_float4(0.f, 0.f, 0.f, 0.f);
+          if (FULL) av = *reinterpret_cast<const float4*>(a_t + soff + c * WG2_KT);
+          else av = (ti + c < Ci) ? *reinterpret_cast<const float4*>(a_s + (ti + c) * WG2_KT) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
           for (int r = 0; r < T; ++r) {
             acc[r][c] = fmaf(dv[r].x, av.x, acc[r][c]);
@@ -494,13 +435,13 @@ wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a,
     if (DGRAD) {
       const int px = 2 * (int)threadIdx.x;       // 256 consumer threads x 2 pixels = one slab
       if (px < left) {                            // `left` is a multiple of 4
-        const long k0 = (slab - b * slabs_per_sample) * KT2;
-        const float* dsp = sm + (size_t)stage * rows * KT2 + px;
+        const long k0 = (slab - b * slabs_per_sample) * WG2_KT;
+        const float* dsp = sm + (size_t)stage * rows * WG2_KT + px;
         float2 o2[2 * T];
 #pragma unroll
         for (int i = 0; i < 2 * T; ++i) o2[i] = make_float2(0.f, 0.f);
         for (int o = 0; o < Co; ++o) {
-          const float2 d = *reinterpret_cast<const float2*>(dsp + (size_t)o * KT2);
+          const float2 d = *reinterpret_cast<const float2*>(dsp + (size_t)o * WG2_KT);
           const float4* wrow = reinterpret_cast<const float4*>(ws + o * 2 * T);
 #pragma unroll
           for (int q = 0; q < 2 * T / 4; ++q) {
@@ -519,7 +460,7 @@ wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a,
     }
     __syncwarp();
     if (lane == 0) mbar_arrive(empty + stage);
-    if (!EARLY_REFILL && warp == 0) produce(slab + NST);    // refill the stage just released (waits for the other warps)
+    if (warp == 0) produce(slab + WG2_STAGES);    // refill the stage just released (waits for the other warps)
   }
   if (!has_tile) return;
   // part[(cta * KH + kh)][Co][Ci + 1]
@@ -543,10 +484,10 @@ wgrad2_partial_kernel(const float* __restrict__ ds, const float* __restrict__ a,
 }
 
 // One place that names every instantiation of the TMA-fed kernel: attr_only sets the shared-memory attribute of all of them
-// (once per device), otherwise the one selected by (dgrad, maps, full) is launched.
-template <int T, bool DGRAD, bool TMAP, bool FULL, typename... Args>
+// (once per device), otherwise the one selected by (dgrad, full) is launched.
+template <int T, bool DGRAD, bool FULL, typename... Args>
 void wg2_launch_one(bool attr_only, dim3 grid, int threads, size_t smem, cudaStream_t st, int& rc, Args... args) {
-  auto kern = wgrad2_partial_kernel<T, DGRAD, WG2_KT, WG2_STAGES, TMAP, TMAP, FULL>;
+  auto kern = wgrad2_partial_kernel<T, DGRAD, FULL>;
   if (attr_only) {
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess)
       rc = check_launch("cudaFuncSetAttribute(wgrad2)");
@@ -555,14 +496,12 @@ void wg2_launch_one(bool attr_only, dim3 grid, int threads, size_t smem, cudaStr
   kern<<<grid, threads, smem, st>>>(args...);
 }
 template <int T, typename... Args>
-void wg2_launch(bool attr_only, bool dgrad, bool maps, bool full, dim3 grid, int threads, size_t smem, cudaStream_t st, int& rc,
+void wg2_launch(bool attr_only, bool dgrad, bool full, dim3 grid, int threads, size_t smem, cudaStream_t st, int& rc,
                 Args... args) {
-  if (attr_only || (dgrad && maps && full)) wg2_launch_one<T, true, true, true>(attr_only, grid, threads, smem, st, rc, args...);
-  if (attr_only || (dgrad && maps && !full)) wg2_launch_one<T, true, true, false>(attr_only, grid, threads, smem, st, rc, args...);
-  if (attr_only || (dgrad && !maps)) wg2_launch_one<T, true, false, false>(attr_only, grid, threads, smem, st, rc, args...);
-  if (attr_only || (!dgrad && maps && full)) wg2_launch_one<T, false, true, true>(attr_only, grid, threads, smem, st, rc, args...);
-  if (attr_only || (!dgrad && maps && !full)) wg2_launch_one<T, false, true, false>(attr_only, grid, threads, smem, st, rc, args...);
-  if (attr_only || (!dgrad && !maps)) wg2_launch_one<T, false, false, false>(attr_only, grid, threads, smem, st, rc, args...);
+  if (attr_only || (dgrad && full)) wg2_launch_one<T, true, true>(attr_only, grid, threads, smem, st, rc, args...);
+  if (attr_only || (dgrad && !full)) wg2_launch_one<T, true, false>(attr_only, grid, threads, smem, st, rc, args...);
+  if (attr_only || (!dgrad && full)) wg2_launch_one<T, false, true>(attr_only, grid, threads, smem, st, rc, args...);
+  if (attr_only || (!dgrad && !full)) wg2_launch_one<T, false, false>(attr_only, grid, threads, smem, st, rc, args...);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -571,7 +510,7 @@ void wg2_launch(bool attr_only, bool dgrad, bool maps, bool full, dim3 grid, int
 // CTA owns the WHOLE 64 x 64 output: 4 pixel groups x 64 threads, thread = 8 x 8 register tile (rows og + 8 j, columns
 // ig + 8 j: consecutive threads touch consecutive shared-memory rows, whose 272-byte pitch spreads them over all banks), 16
 // LDS.128 per 256 FMA, slabs of 64 pixels through a 2-stage cp.async ring, two CTAs per SM.  The pixel groups are summed
-// through shared memory at the end; per-CTA partials go through wgrad_reduce_kernel like the other forms.
+// through shared memory at the end; per-CTA partials go through partial_reduce_kernel like the other forms.
 // ------------------------------------------------------------------------------------------
 constexpr int WW_KT = 64;          // pixels per slab
 constexpr int WW_P = WW_KT + 4;    // row pitch (floats)
@@ -677,37 +616,9 @@ wgrad_wide_kernel(const float* __restrict__ ds, const float* __restrict__ a, flo
   if (tid < Co) pp[(size_t)tid * (Ci + 1) + Ci] = (redb[4 * tid] + redb[4 * tid + 1]) + (redb[4 * tid + 2] + redb[4 * tid + 3]);
 }
 
-// one warp per output element: lanes stride the per-CTA partials, fixed-order shuffle tree
-__global__ void __launch_bounds__(128)
-wgrad_reduce_kernel(const float* __restrict__ part, float* __restrict__ gW, float* __restrict__ gb, int nparts,
-                    int Co, int Ci) {
-  const int idx = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  const int total = Co * (Ci + 1);
-  if (idx >= total) return;
-  float s = 0.f;
-  for (int p = lane; p < nparts; p += 32) s += part[(size_t)p * total + idx];
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
-  if (lane != 0) return;
-  const int o = idx / (Ci + 1), i = idx - o * (Ci + 1);
-  if (i < Ci) {
-    if (gW != nullptr) gW[(size_t)o * Ci + i] = s;
-  } else if (gb != nullptr) {
-    gb[o] = s;
-  }
-}
-
 constexpr int WG_CTAS = 148 * 2;  // persistent grid: 2 resident CTAs per SM (register-limited)
 
 }  // namespace
-
-int launch_wgrad_reduce(const float* part, float* gW, float* gb, int nparts, int Co, int Ci, cudaStream_t st) {
-  const int total = Co * (Ci + 1);
-  wgrad_reduce_kernel<<<(total * 32 + 127) / 128, 128, 0, st>>>(part, gW, gb, nparts, Co, Ci);
-  count_launch();
-  return check_launch("wgrad_reduce_kernel");
-}
 }  // namespace fno
 
 using namespace fno;
@@ -780,10 +691,16 @@ static int pointwise_wgrad_impl(const float* ds, const float* a, float* gW, floa
   ctas = (total_slabs + spc - 1) / spc;
   const int aligned = (N % 4 == 0) && ((reinterpret_cast<size_t>(ds) | reinterpret_cast<size_t>(a)) % 16 == 0);
   float* part = static_cast<float*>(work);
-  dim3 grid((unsigned)ctas, ygroups);
-  // v2 (TMA bulk-fed): persistent CTAs, one per SM, each over a contiguous range of 512-pixel slabs
+  int nparts = 0;
+  // v2 (TMA-fed): persistent CTAs, one per SM, each over a contiguous range of 512-pixel slabs; the operand feed is two 2-D
+  // tensor-map copies per slab (box {512 pixels as 256 8-byte elements, C planes} of ds and of a)
   const size_t smem2 = sizeof(float) * (size_t)WG2_STAGES * (Co + Ci) * WG2_KT + 2 * WG2_STAGES * sizeof(unsigned long long);
-  if (aligned && smem2 <= 200 * 1024 && ntiles <= WG2_MAXW) {
+  CUtensorMap mds, ma;
+  memset(&mds, 0, sizeof(mds)); memset(&ma, 0, sizeof(ma));
+  const auto l2 = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+  if (aligned && smem2 <= 200 * 1024 && ntiles <= WG2_MAXW && N < (1L << 31) && (long)B * (Co > Ci ? Co : Ci) < (1L << 31) &&
+      make_plane_map(&mds, ds, (unsigned long long)N, (unsigned long long)B * Co, WG2_KT, Co, 8, l2) &&
+      make_plane_map(&ma, a, (unsigned long long)N, (unsigned long long)B * Ci, WG2_KT, Ci, 8, l2)) {
     const int KH = (2 * ntiles <= WG2_MAXW) ? 2 : 1;       // pixel halves per tile
     const int warps2 = ntiles * KH;
     const int sps2 = (int)((N + WG2_KT - 1) / WG2_KT);
@@ -795,47 +712,29 @@ static int pointwise_wgrad_impl(const float* ds, const float* a, float* gW, floa
     const size_t smem2d = smem2 + sizeof(float) * (size_t)Co * 2 * T;
     const bool dgrad = Wm != nullptr && dx != nullptr && warps2 == WG2_MAXW && Co <= 2 * T && Ci <= 2 * T &&
                        smem2d <= 200 * 1024 && (reinterpret_cast<size_t>(dx) % 8) == 0;
-    // operand feed: two 2-D tensor-map copies per slab (box {512 pixels as 256 8-byte elements, C planes} of ds and of a)
-    // when the driver entry point is there, else one bulk copy per channel row (FNO_WG2=0 forces the latter)
-    CUtensorMap mds, ma;
-    memset(&mds, 0, sizeof(mds)); memset(&ma, 0, sizeof(ma));
-    const bool use_map = wg2_use_maps() && N < (1L << 31) && (long)B * (Co > Ci ? Co : Ci) < (1L << 31) &&
-                         wg2_make_map(&mds, ds, (unsigned long long)N, (unsigned long long)B * Co, WG2_KT, Co) &&
-                         wg2_make_map(&ma, a, (unsigned long long)N, (unsigned long long)B * Ci, WG2_KT, Ci);
-    const bool full = use_map && (T % 2 == 0) && tiles_i == 2 && Ci == 2 * T && Co % T == 0;
+    const bool full = (T % 2 == 0) && tiles_i == 2 && Ci == 2 * T && Co % T == 0;
     static PerDeviceOnce attr2_done;
     if (attr2_done.need()) {
       int rca = FNO_OK;
-      wg2_launch<T>(true, true, true, true, dim3(1), 0, 0, st, rca, ds, a, part, Co, Ci, N, sps2, total2s, spc2, tiles_i, ntiles,
+      wg2_launch<T>(true, true, true, dim3(1), 0, 0, st, rca, part, Co, Ci, N, sps2, total2s, spc2, tiles_i, ntiles,
                     warps2, KH, Wm, dx, mds, ma);
       if (rca != FNO_OK) return rca;
       attr2_done.mark();
     }
     int rcl = FNO_OK;
-    wg2_launch<T>(false, dgrad, use_map, full, dim3((unsigned)ctas2, 1), 32 * warps2, dgrad ? smem2d : smem2, st, rcl, ds, a, part,
-                  Co, Ci, N, sps2, total2s, spc2, tiles_i, ntiles, warps2, KH, dgrad ? Wm : nullptr, dgrad ? dx : nullptr, mds, ma);
+    wg2_launch<T>(false, dgrad, full, dim3((unsigned)ctas2, 1), 32 * warps2, dgrad ? smem2d : smem2, st, rcl, part, Co,
+                  Ci, N, sps2, total2s, spc2, tiles_i, ntiles, warps2, KH, dgrad ? Wm : nullptr, dgrad ? dx : nullptr, mds, ma);
     if (rcl != FNO_OK) return rcl;
-    const long nparts2 = ctas2 * KH;
     if (dgrad && fused) *fused = 1;
     count_launch();
     int rc2 = check_launch("wgrad2_partial_kernel");
     if (rc2 != FNO_OK) return rc2;
-    const int total2 = Co * (Ci + 1);
-    wgrad_reduce_kernel<<<(total2 * 32 + 127) / 128, 128, 0, st>>>(part, gW, gb, (int)nparts2, Co, Ci);
-    count_launch();
-    return check_launch("wgrad_reduce_kernel");
-  }
-  if (aligned && pointwise_tc_supported(Ci, Co)) {
+    nparts = (int)(ctas2 * KH);
+  } else if (aligned && pointwise_tc_supported(Ci, Co)) {
     // wide channels on tcgen05: [ds ; a] [a ; 1]^T per 64-pixel slab, accumulator in TMEM (pointwise_tc.cu)
-    int nparts = 0;
     int rct = launch_wgrad_tc(ds, a, part, B, Co, Ci, N, WG_CTAS, &nparts, st);
     if (rct != FNO_OK) return rct;
-    const int totalo = Co * (Ci + 1);
-    wgrad_reduce_kernel<<<(totalo * 32 + 127) / 128, 128, 0, st>>>(part, gW, gb, nparts, Co, Ci);
-    count_launch();
-    return check_launch("wgrad_reduce_kernel");
-  }
-  if (aligned && ygroups > 1 && Co <= WW_C && Ci <= WW_C) {
+  } else if (aligned && ygroups > 1 && Co <= WW_C && Ci <= WW_C) {
     // wide channels: one CTA owns the whole Co x Ci output (wgrad_wide_kernel)
     const size_t smemw = sizeof(float) * 2ul * 2 * WW_C * WW_P;
     static_assert(sizeof(float) * (4ul * WW_C * WW_C + WW_THREADS) <= sizeof(float) * 2ul * 2 * WW_C * WW_P, "reduce buffer fits the ring");
@@ -854,20 +753,21 @@ static int pointwise_wgrad_impl(const float* ds, const float* a, float* gW, floa
     count_launch();
     int rcw = check_launch("wgrad_wide_kernel");
     if (rcw != FNO_OK) return rcw;
-    const int totalo = Co * (Ci + 1);
-    wgrad_reduce_kernel<<<(totalo * 32 + 127) / 128, 128, 0, st>>>(part, gW, gb, (int)ctasw, Co, Ci);
+    nparts = (int)ctasw;
+  } else {
+    const dim3 grid((unsigned)ctas, ygroups);
+    wgrad_partial_kernel<T><<<grid, 32 * warps, smem, st>>>(ds, a, part, Co, Ci, N, slabs_per_sample, total_slabs, spc,
+                                                          tiles_i, ntiles, aligned);
     count_launch();
-    return check_launch("wgrad_reduce_kernel");
+    int rc = check_launch("wgrad_partial_kernel");
+    if (rc != FNO_OK) return rc;
+    nparts = (int)ctas;
   }
-  wgrad_partial_kernel<T><<<grid, 32 * warps, smem, st>>>(ds, a, part, Co, Ci, N, slabs_per_sample, total_slabs, spc,
-                                                        tiles_i, ntiles, aligned);
-  count_launch();
-  int rc = check_launch("wgrad_partial_kernel");
-  if (rc != FNO_OK) return rc;
-  const int total = Co * (Ci + 1);
-  wgrad_reduce_kernel<<<(total * 32 + 127) / 128, 128, 0, st>>>(part, gW, gb, (int)ctas, Co, Ci);
-  count_launch();
-  return check_launch("wgrad_reduce_kernel");
+  // records [nparts][Co][Ci + 1]: gW in the first Ci columns, gb in the last
+  ReduceSegs segs;
+  segs.s[0] = {gW, Co * Ci, 0, Ci, Ci + 1};
+  segs.s[1] = {gb, Co, Ci, 1, Ci + 1};
+  return launch_partial_reduce(part, nparts, Co * (Ci + 1), segs, st);
 }
 
 extern "C" int fno_pointwise_wgrad(const float* ds, const float* a, float* gW, float* gb, void* work, int B, int Co,

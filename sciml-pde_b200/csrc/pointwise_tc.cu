@@ -201,7 +201,7 @@ pointwise_tc_kernel(const float* __restrict__ in, const float* __restrict__ W, c
 // The tensor core's fp32 accumulate truncates: a chain of ~500 MMAs into one TMEM tile measured 7e-6 of relative error
 // (biased, so it grows with the chain), too much for the 1e-5 fp32-mode bound.  A TMEM tile therefore only collects
 // WT_CHAIN = 2 slabs (48 MMAs); the loader warps drain it into IEEE fp32 register accumulators while the next chain fills
-// the other tile.  Per-CTA partials go through wgrad_reduce_kernel.
+// the other tile.  Per-CTA partials go through partial_reduce_kernel.
 // ------------------------------------------------------------------------------------------
 // RA = rows of the gradient (64: the bypass; 128: the projection head's hidden layer, head_wide_tc.cu -- then A is the
 // ds block alone and B = [a ; 1]), KT = pixels per slab (64 / 32: the stacked buffer must fit twice, hi and lo).
@@ -411,7 +411,7 @@ int launch_pointwise_tc(const float* in, const float* W, const float* bias, floa
   return check_launch("pointwise_tc_kernel");
 }
 
-// per-CTA partial records [ctas][Co][Ci + 1] into `part` (the caller runs wgrad_reduce_kernel over them); returns the
+// per-CTA partial records [ctas][Co][Ci + 1] into `part` (the caller runs partial_reduce_kernel over them); returns the
 // number of records through *nparts.  Needs N % 4 == 0 and 16-byte aligned tensors (the caller checks).
 template <int RA, int KT>
 static int launch_wgrad_tc_t(const float* ds, const float* a, float* part, int B, int Co, int Ci, long N, int max_parts,

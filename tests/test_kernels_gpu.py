@@ -310,9 +310,9 @@ def test_mix_tensor_core_math_modes(lib, low):
     (3, 8, 8, (13, 11)),         # N not a multiple of 4 -> scalar path
     (2, 6, 10, (16, 16)),        # Co != Ci
     (1, 64, 64, (66, 66)),
-    (3, 64, 64, (258, 258)),     # cfg-3 planes: wide-channel weight gradient (one CTA owns the 64 x 64 output), ragged last slab
+    (3, 64, 64, (258, 258)),     # cfg-3 planes: tcgen05 weight gradient (wgrad_tc_kernel<64, 64>), ragged last slab
     (2, 48, 33, (30, 34)),       # wide, Co != Ci, channel counts that are not multiples of 8
-    (2, 24, 24, (20, 20)),
+    (2, 24, 24, (20, 20)),       # FP32 wide-channel weight gradient (one CTA owns the whole output)
     (2, 20, 20, (16, 16, 22)),
     (1, 5, 3, (9, 7)),           # channel counts that are not tile multiples
 ])

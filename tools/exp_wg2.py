@@ -1,9 +1,7 @@
 #!/usr/bin/env python
 """Bypass weight gradient (csrc/pointwise.cu, wgrad2_partial_kernel) at the cfg-1 layer geometry: parity against an fp64 einsum on
-ragged cases (with and without the fused data gradient), then event-timed launches with L2 flushed in between.  The operand
-feed is chosen once per process: FNO_WG2=0 python tools/exp_wg2.py times the bulk-copy form, the default the tensor-map form
-(profiles/r2g_wgrad_forms.md has the sweep over ring shapes that led there)."""
-import os
+ragged cases (with and without the fused data gradient), then event-timed launches with L2 flushed in between
+(profiles/r2g_wgrad_forms.md has the sweep over operand feeds and ring shapes that led to the tensor-map feed)."""
 import sys
 from pathlib import Path
 
@@ -25,7 +23,7 @@ def ref(ds, a):
     return torch.einsum("bop,bip->oi", d64, a64), d64.sum((0, 2))
 
 
-def check(form, B, C, n):
+def check(B, C, n):
     ds = torch.randn(B, C, n, n, device=dev)
     a = torch.randn(B, C, n, n, device=dev) + 0.5
     gw, gb = lib.pointwise_wgrad(ds, a, (C, C, 1, 1))
@@ -35,7 +33,7 @@ def check(form, B, C, n):
     return ew, eb
 
 
-def timeit(form, B, C, n, iters=20):
+def timeit(B, C, n, iters=20):
     ds = torch.randn(B, C, n, n, device=dev)
     a = torch.randn(B, C, n, n, device=dev)
     bufs = lib.pointwise_wgrad_buffers(ds, a, (C, C, 1, 1))
@@ -56,10 +54,9 @@ def timeit(form, B, C, n, iters=20):
     return med, ts[0], nbytes / med * 1e-3
 
 
-form = os.environ.get("FNO_WG2", "default")
 for (B, C, n) in ((3, 20, 34), (2, 12, 130), (5, 20, 66), (16, 20, 130), (2, 30, 34), (2, 8, 66)):
-    ew, eb = check(form, B, C, n)
-    print(f"form {form} parity B={B} C={C} n={n}: gW {ew:.2e} gb {eb:.2e}", "OK" if max(ew, eb) < 1e-5 else "FAIL", flush=True)
+    ew, eb = check(B, C, n)
+    print(f"parity B={B} C={C} n={n}: gW {ew:.2e} gb {eb:.2e}", "OK" if max(ew, eb) < 1e-5 else "FAIL", flush=True)
 # the fused data gradient (cfg 4's unfused layers): dx = W^T ds from the same slabs
 for (B, C, n) in ((3, 20, 34), (4, 20, 130), (2, 12, 66)):
     ds = torch.randn(B, C, n, n, device=dev)
@@ -70,7 +67,7 @@ for (B, C, n) in ((3, 20, 34), (4, 20, 130), (2, 12, 66)):
     rw, rb = ref(ds, a)
     e = [float((dx.double() - rdx).abs().max() / rdx.abs().max()), float((gw.double().view(C, C) - rw).abs().max() / rw.abs().max()),
          float((gb.double() - rb).abs().max() / rb.abs().max())]
-    print(f"form {form} bwd (dgrad) B={B} C={C} n={n}: dx {e[0]:.2e} gW {e[1]:.2e} gb {e[2]:.2e}", "OK" if max(e) < 1e-5 else "FAIL", flush=True)
+    print(f"bwd (dgrad) B={B} C={C} n={n}: dx {e[0]:.2e} gW {e[1]:.2e} gb {e[2]:.2e}", "OK" if max(e) < 1e-5 else "FAIL", flush=True)
 for B in (128, 32):
-    med, best, gbs = timeit(form, B, 20, 130)
-    print(f"form {form} B={B}: median {med:.1f} us, best {best:.1f} us, {gbs:.0f} GB/s (wgrad2 + reduce)", flush=True)
+    med, best, gbs = timeit(B, 20, 130)
+    print(f"B={B}: median {med:.1f} us, best {best:.1f} us, {gbs:.0f} GB/s (wgrad2 + reduce)", flush=True)
