@@ -186,12 +186,21 @@ int fno_lift_stats(const float* x, float* stats, void* work, int B, long entries
 int fno_lift_fwd(const float* x, const float* grid, const float* stats, const float* W0,
                  const float* b0, float* h, int B, int R_in, int W_in, int R_out, int Wp, int T,
                  int V, int G, int C, fno_stream_t stream);
-/* autograd backward of the above w.r.t. fc0: gW0 [C, T*V+G], gb0 [C] from dh [B, C, R_out, Wp]
- * (the model input and the statistics carry no gradient, fno/fno.py:140).                          */
+/* autograd backward of the above w.r.t. fc0: gW0 [C, T*V+G], gb0 [C] from dh [B, C, R_out, Wp].
+ * Only the statistics are constants (computed under no_grad, fno/fno.py:140-142); the gradient
+ * w.r.t. the model input is fno_lift_dgrad.                                                       */
 size_t fno_lift_bwd_workspace_bytes(int T, int V, int G, int C);
 int fno_lift_bwd(const float* x, const float* grid, const float* stats, const float* dh, float* gW0,
                  float* gb0, void* work, int B, int R_in, int W_in, int R_out, int Wp, int T, int V,
                  int G, int C, fno_stream_t stream);
+/* autograd backward of fno_lift_fwd w.r.t. its data inputs, the statistics held constant:
+ *   dx [B, R_in*W_in, T, V]:  dx[b,p,t,v] = (1 / stats[b,1,v]) sum_c W0[c, t*V+v] dh[b, c, off(p)]
+ *   dgrid [B, R_in*W_in, G]:  dgrid[b,p,g] = sum_c W0[c, T*V+g] dh[b, c, off(p)]
+ * Only the valid region of dh is read.  Either output may be NULL (not both); 1 <= V <= 8.
+ * No workspace.                                                                                     */
+int fno_lift_dgrad(const float* dh, const float* W0, const float* stats, float* dx, float* dgrid,
+                   int B, int R_in, int W_in, int R_out, int Wp, int T, int V, int G, int C,
+                   fno_stream_t stream);
 
 /* ---- projection head: unpad, fc1, exact GELU, fc2, de-normalise (SURVEY 8f row f1) ---------------- */
 /* fno/fno.py:180-187, :381-389.  h [B, C, R_out, Wp] (trunk layout, read in place), W1 [HID, C],
@@ -280,6 +289,11 @@ int fno_metric_func(const float* pred, const float* target, void* work, float* o
  * (metrics.py:344): xx, xx_out [points, T0, V], pred [points, 1, V]; xx_out != xx. */
 int fno_window_shift(const float* xx, const float* pred, float* xx_out, long points, int T0, int V,
                      fno_stream_t stream);
+/* Its adjoint, for training through a rollout: g [points, T0, V] -> gxx [points, T0, V] with
+ * gxx[.., 0, :] = 0 and gxx[.., t, :] = g[.., t-1, :], and gpred [points, 1, V] = g[.., T0-1, :].
+ * Either output may be NULL (not both); gxx != g.                                                   */
+int fno_window_shift_bwd(const float* g, float* gxx, float* gpred, long points, int T0, int V,
+                         fno_stream_t stream);
 
 /* ---- step tail: loss, gradient clipping, Adam, LR schedule (SURVEY 8f row f3) --------------------- */
 /* nrmse(out, target).mean() of fno/train.py:34-40,:266-267 for out / target [B, P, V] (P = pixels x

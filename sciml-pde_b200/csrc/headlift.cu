@@ -4,7 +4,8 @@
 //
 //   lift  (fno/fno.py:140-159, :343-360): per-sample statistics -> normalise -> [x_tv, grid] ->
 //         fc0 -> NCHW -> zero pad, written straight into the trunk layout (no cat / permute /
-//         pad tensors); backward = fc0 weight/bias gradient only (the input needs no gradient).
+//         pad tensors); backward = fc0 weight/bias gradient, and the gradient w.r.t. x and grid when
+//         they need one (only the statistics are constants, as under the reference's no_grad).
 //   head  (fno/fno.py:180-188, :381-390): unpad -> NHWC -> fc1 -> exact GELU -> fc2 ->
 //         de-normalise, reading the padded layout in place.  The 128-wide hidden layer
 //         (8.4 MB/sample at 128x128) never exists in memory: forward keeps it in registers,
@@ -570,6 +571,96 @@ lift_bwd2_kernel(const float* __restrict__ x, const float* __restrict__ grid, co
     const int f_q = item / CQ, c_q = item - f_q * CQ;
     const int c = 4 * c_q + a, f = 4 * f_q + bb;
     if (c < C && f <= F) pp[(size_t)c * (F + 1) + f] = sum;
+  }
+}
+
+// ------------------------------------------------------------------------------------------
+// lift data gradient (the statistics are constants, as under the reference's no_grad):
+//   dx[b, p, t, v]  = (1 / sd[b, v]) sum_c W0[c, t V + v] dh[b, c, off(p)]
+//   dgrid[b, p, g]  =                sum_c W0[c, T V + g] dh[b, c, off(p)]
+// One CTA per 64-pixel row tile.  Only the valid columns of dh are read: whatever the adjoint of the first layer left in
+// the padding never reaches dx.  Item = (feature quad, pixel pair): lanes over the 32 pixel pairs read a channel row of
+// the tile as one 256-byte line, warps over quads read the W0 quad as a broadcast (2 shared loads per 8 FMAs).  The
+// result goes through a feature-major tile in shared memory, because the tile's dx block is contiguous in HBM
+// (nv * T * V floats): it leaves as coalesced 16-byte stores instead of per-pixel stores at a T * V * 4-byte lane stride.
+// ------------------------------------------------------------------------------------------
+constexpr int LD_THREADS = 256;
+constexpr int LD_OP = TILE + 1;           // output-tile pitch: the transposing read of a warp spreads over the banks
+
+size_t lift_dgrad_smem(int C, int F) {
+  const int FR = 4 * ((F + 3) / 4);
+  return sizeof(float) * ((size_t)C * FR + (size_t)C * TILE + (size_t)FR * LD_OP);
+}
+
+__global__ void __launch_bounds__(LD_THREADS)
+lift_dgrad_kernel(const float* __restrict__ dh, const float* __restrict__ W0, const float* __restrict__ stats,
+                  float* __restrict__ dx, float* __restrict__ dgrid, PixGeo g, TileMap tm, int T, int V, int G, int C,
+                  int q0, int q1) {
+  extern __shared__ __align__(16) float sm[];
+  const int F1 = T * V, F = F1 + G, FR = 4 * ((F + 3) / 4);
+  float* ws = sm;                             // [C][FR]      W0, zero beyond F
+  float* dhs = ws + (size_t)C * FR;           // [C][TILE]    the tile's dh rows, zero beyond the valid columns
+  float* os = dhs + (size_t)C * TILE;         // [FR][LD_OP]  dx | dgrid of the tile, feature-major
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int b, r, w0;
+  decode_tile(tm, g, blockIdx.x, b, r, w0);
+  const int nv = min(TILE, g.W_in - w0);
+  for (int i = tid; i < C * FR; i += LD_THREADS) {
+    const int c = i / FR, f = i - c * FR;
+    ws[i] = f < F ? __ldg(W0 + (size_t)c * F + f) : 0.f;
+  }
+  {
+    const int k = tid & (TILE - 1);
+    const float* __restrict__ dp = dh + (size_t)b * C * g.plane + (size_t)r * g.Wp + w0 + k;
+#pragma unroll 4
+    for (int c = tid / TILE; c < C; c += LD_THREADS / TILE) dhs[c * TILE + k] = k < nv ? __ldg(dp + (size_t)c * g.plane) : 0.f;
+  }
+  __syncthreads();
+  const float* __restrict__ sd = stats + (size_t)b * 2 * V + V;
+  for (int q = q0 + warp; q < q1; q += LD_THREADS / 32) {
+    float a0[4] = {0.f, 0.f, 0.f, 0.f}, a1[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 4
+    for (int c = 0; c < C; ++c) {
+      const float2 d = *reinterpret_cast<const float2*>(dhs + c * TILE + 2 * lane);
+      const float4 w = *reinterpret_cast<const float4*>(ws + c * FR + 4 * q);
+      a0[0] = fmaf(w.x, d.x, a0[0]); a0[1] = fmaf(w.y, d.x, a0[1]); a0[2] = fmaf(w.z, d.x, a0[2]); a0[3] = fmaf(w.w, d.x, a0[3]);
+      a1[0] = fmaf(w.x, d.y, a1[0]); a1[1] = fmaf(w.y, d.y, a1[1]); a1[2] = fmaf(w.z, d.y, a1[2]); a1[3] = fmaf(w.w, d.y, a1[3]);
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int f = 4 * q + j;
+      if (f < F) {
+        const float s = f < F1 ? 1.0f / __ldg(sd + f % V) : 1.0f;   // the forward's reciprocal of std + 1e-7
+        os[f * LD_OP + 2 * lane] = a0[j] * s;
+        os[f * LD_OP + 2 * lane + 1] = a1[j] * s;
+      }
+    }
+  }
+  __syncthreads();
+  const size_t p0 = (size_t)b * g.npix + (size_t)r * g.W_in + w0;   // first pixel of the tile
+  if (dx != nullptr) {
+    float* __restrict__ out = dx + p0 * F1;
+    const int n = nv * F1;
+    if ((F1 & 3) == 0 && (reinterpret_cast<size_t>(out) & 15) == 0) {
+      for (int i = 4 * tid; i < n; i += 4 * LD_THREADS) {
+        const int k = i / F1, f = i - k * F1;
+        const float* o = os + f * LD_OP + k;
+        *reinterpret_cast<float4*>(out + i) = make_float4(o[0], o[LD_OP], o[2 * LD_OP], o[3 * LD_OP]);
+      }
+    } else {
+      for (int i = tid; i < n; i += LD_THREADS) {
+        const int k = i / F1, f = i - k * F1;
+        out[i] = os[f * LD_OP + k];
+      }
+    }
+  }
+  if (dgrid != nullptr && G > 0) {
+    float* __restrict__ out = dgrid + p0 * G;
+    const int n = nv * G;
+    for (int i = tid; i < n; i += LD_THREADS) {
+      const int k = i / G, f = i - k * G;
+      out[i] = os[(F1 + f) * LD_OP + k];
+    }
   }
 }
 
@@ -1156,6 +1247,33 @@ extern "C" int fno_lift_bwd(const float* x, const float* grid, const float* stat
   segs.s[0] = {gW0, C * F, 0, F, F + 1};
   segs.s[1] = {gb0, C, F, 1, F + 1};
   return launch_partial_reduce(part, ctas * KSPL, C * (F + 1), segs, st);
+}
+
+extern "C" int fno_lift_dgrad(const float* dh, const float* W0, const float* stats, float* dx, float* dgrid, int B,
+                              int R_in, int W_in, int R_out, int Wp, int T, int V, int G, int C, fno_stream_t stream) {
+  if (!dh || !W0 || !stats || (!dx && !dgrid) || bad_geo(B, R_in, W_in, R_out, Wp) || T < 1 || V < 1 || V > VMAX ||
+      G < 0 || C < 1) {
+    set_error("fno_lift_dgrad: bad argument (need dx or dgrid, 1 <= V <= %d)", VMAX);
+    return FNO_E_ARG;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const PixGeo g = make_geo(R_in, W_in, R_out, Wp);
+  const int F1 = T * V, F = F1 + G;
+  const size_t smem = lift_dgrad_smem(C, F);
+  if (smem > 160 * 1024) { set_error("fno_lift_dgrad: %d channels x %d features do not fit shared memory", C, F); return FNO_E_ARG; }
+  const TileMap tm = make_tiles(g, B);
+  if (tm.total <= 0) { set_error("fno_lift_dgrad: too many pixel tiles"); return FNO_E_ARG; }
+  static PerDeviceOnce done;
+  if (done.need()) {
+    if (cudaFuncSetAttribute(lift_dgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024) != cudaSuccess)
+      return check_launch("cudaFuncSetAttribute(lift_dgrad)");
+    done.mark();
+  }
+  // feature quads to compute: those holding dx features and / or grid features
+  const int q0 = dx ? 0 : F1 / 4, q1 = dgrid ? (F + 3) / 4 : (F1 + 3) / 4;
+  lift_dgrad_kernel<<<tm.total, LD_THREADS, smem, st>>>(dh, W0, stats, dx, dgrid, g, tm, T, V, G, C, q0, q1);
+  count_launch();
+  return check_launch("lift_dgrad_kernel");
 }
 
 extern "C" int fno_head_fwd(const float* h, const float* W1, const float* b1, const float* W2, const float* b2,

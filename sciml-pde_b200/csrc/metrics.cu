@@ -238,6 +238,20 @@ window_shift_kernel(const float* __restrict__ xx, const float* __restrict__ pred
   }
 }
 
+// its adjoint: gxx[..., 0, :] = 0, gxx[..., t, :] = g[..., t - 1, :], gpred = g[..., T0 - 1, :] (either output may be null)
+__global__ void __launch_bounds__(256)
+window_shift_bwd_kernel(const float* __restrict__ g, float* __restrict__ gxx, float* __restrict__ gpred, long points,
+                        int T0, int V) {
+  const long total = points * T0 * V;
+  const int TV = T0 * V;
+  for (long o = (long)blockIdx.x * blockDim.x + threadIdx.x; o < total; o += (long)gridDim.x * blockDim.x) {
+    const long pt = o / TV;
+    const int e = (int)(o - pt * TV);
+    if (gxx != nullptr) gxx[o] = e < V ? 0.f : __ldg(g + o - V);
+    if (gpred != nullptr && e >= TV - V) gpred[pt * V + (e - (TV - V))] = __ldg(g + o);
+  }
+}
+
 size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
 
 struct MetricWork {
@@ -351,4 +365,16 @@ extern "C" int fno_window_shift(const float* xx, const float* pred, float* xx_ou
                                                                                               T0, V);
   count_launch();
   return check_launch("window_shift_kernel");
+}
+
+extern "C" int fno_window_shift_bwd(const float* g, float* gxx, float* gpred, long points, int T0, int V,
+                                    fno_stream_t stream) {
+  if (!g || (!gxx && !gpred) || points <= 0 || T0 <= 0 || V <= 0 || g == gxx) {
+    set_error("fno_window_shift_bwd: bad argument (need gxx or gpred; in-place is not supported)");
+    return FNO_E_ARG;
+  }
+  window_shift_bwd_kernel<<<grid_for(points * T0 * V), 256, 0, static_cast<cudaStream_t>(stream)>>>(g, gxx, gpred,
+                                                                                                    points, T0, V);
+  count_launch();
+  return check_launch("window_shift_bwd_kernel");
 }

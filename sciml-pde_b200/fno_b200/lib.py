@@ -61,6 +61,7 @@ def load():
             "fno_metric_workspace_bytes": (C.c_size_t, [i, i, i, i, i, i]),
             "fno_metric_func": (i, [vp, vp, vp, vp, i, i, i, i, i, i, f, f, f, i, i, vp]),
             "fno_window_shift": (i, [vp, vp, vp, l, i, i, vp]),
+            "fno_window_shift_bwd": (i, [vp, vp, vp, l, i, i, vp]),
             "fno_set_math_mode": (i, [i]),
             "fno_get_math_mode": (i, []),
             "fno_plan_destroy": (i, [vp]),
@@ -86,6 +87,7 @@ def load():
             "fno_lift_fwd": (i, [vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i, i, i, vp]),
             "fno_lift_bwd_workspace_bytes": (C.c_size_t, [i, i, i, i]),
             "fno_lift_bwd": (i, [vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i, i, i, vp]),
+            "fno_lift_dgrad": (i, [vp, vp, vp, vp, vp, i, i, i, i, i, i, i, i, i, vp]),
             "fno_head_fwd": (i, [vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i, i, vp]),
             "fno_head_fwd_tc": (i, [vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i, i, vp]),
             "fno_head_bwd_workspace_bytes": (C.c_size_t, [i, i, i]),
@@ -124,11 +126,11 @@ EXPORTED_SYMBOLS = (
     "fno_layer2d_fused_workspace_bytes", "fno_layer2d_inv_fused", "fno_pointwise_fwd",
     "fno_pointwise_wgrad_workspace_bytes", "fno_pointwise_wgrad", "fno_pointwise_bwd",
     "fno_lift_stats_workspace_bytes", "fno_lift_stats", "fno_lift_fwd", "fno_lift_bwd_workspace_bytes",
-    "fno_lift_bwd", "fno_head_fwd", "fno_head_fwd_tc", "fno_head_bwd_workspace_bytes", "fno_head_bwd", "fno_head_bwd_tc",
+    "fno_lift_bwd", "fno_lift_dgrad", "fno_head_fwd", "fno_head_fwd_tc", "fno_head_bwd_workspace_bytes", "fno_head_bwd", "fno_head_bwd_tc",
     "fno_head_fwd_wide_tc", "fno_head_bwd_wide_supported", "fno_head_bwd_wide_workspace_bytes", "fno_head_bwd_wide_tc",
     "fno_nrmse_workspace_bytes", "fno_nrmse_fwd", "fno_nrmse_bwd", "fno_opt_chunk_floats",
     "fno_opt_chunk_bytes", "fno_clip_adam_step",
-    "fno_metric_workspace_bytes", "fno_metric_func", "fno_window_shift",
+    "fno_metric_workspace_bytes", "fno_metric_func", "fno_window_shift", "fno_window_shift_bwd",
     "fno_sc1d_fwd_transform", "fno_sc1d_inv_transform", "fno_mix1d_fwd", "fno_mix1d_bwd",
 )
 
@@ -548,6 +550,22 @@ def lift_bwd(geo: TrunkGeo, x, grid, stats, dh, W0_shape):
     return gW0, gb0
 
 
+@_on_tensor_device
+def lift_dgrad(geo: TrunkGeo, dh, W0, stats, x_shape, grid_shape, *, need_dx: bool = True, need_dgrid: bool = False):
+    """Gradient of lift_fwd w.r.t. x [B, *spatial, T, V] and grid [B, *spatial, G] (statistics held constant), from
+    dh in trunk layout.  Returns (dx or None, dgrid or None)."""
+    for t, n in ((dh, "dh"), (W0, "fc0.weight"), (stats, "stats")):
+        _require(t, torch.float32, n)
+    B, T, V, G, C = x_shape[0], x_shape[-2], x_shape[-1], grid_shape[-1], W0.shape[0]
+    if tuple(dh.shape) != (B, C) + geo.padded or W0.shape[1] != T * V + G:
+        raise FnoError(f"lift_dgrad: dh {tuple(dh.shape)} / fc0.weight {tuple(W0.shape)} do not match x {tuple(x_shape)}")
+    dx = torch.empty(tuple(x_shape), dtype=torch.float32, device=dh.device) if need_dx else None
+    dgrid = torch.empty(tuple(grid_shape), dtype=torch.float32, device=dh.device) if need_dgrid else None
+    _check(load().fno_lift_dgrad(dh.data_ptr(), W0.data_ptr(), stats.data_ptr(), _ptr(dx), _ptr(dgrid), B, *geo.ints,
+                                 T, V, G, C, _stream()), "fno_lift_dgrad")
+    return dx, dgrid
+
+
 MATH_MODES = {"fp32": 0, "tf32": 1, "bf16": 2}
 
 
@@ -678,6 +696,18 @@ def window_shift(xx: torch.Tensor, pred: torch.Tensor, out: Optional[torch.Tenso
     _check(load().fno_window_shift(xx.data_ptr(), pred.data_ptr(), out.data_ptr(), points, T0, V, _stream()),
            "fno_window_shift")
     return out
+
+
+@_on_tensor_device
+def window_shift_bwd(g: torch.Tensor, *, need_xx: bool = True, need_pred: bool = True):
+    """Adjoint of window_shift: g [..., T0, V] -> (gxx [..., T0, V] or None, gpred [..., 1, V] or None)."""
+    _require(g, torch.float32, "g")
+    T0, V = g.shape[-2:]
+    gxx = torch.empty_like(g) if need_xx else None
+    gpred = torch.empty(tuple(g.shape[:-2]) + (1, V), dtype=torch.float32, device=g.device) if need_pred else None
+    _check(load().fno_window_shift_bwd(g.data_ptr(), _ptr(gxx), _ptr(gpred), g.numel() // (T0 * V), T0, V, _stream()),
+           "fno_window_shift_bwd")
+    return gxx, gpred
 
 
 # ---- SpectralConv1d ------------------------------------------------------------------------------------------

@@ -143,8 +143,11 @@ def fourier_layer(a, wl, bl, apply_gelu: bool, weights: Sequence[torch.Tensor]) 
 class LiftFn(torch.autograd.Function):
     """h = pad(permute(fc0(cat(normalise(x), grid))))  -- fno/fno.py:140-159, :343-360.
 
-    One kernel writes the trunk layout directly; backward is the fc0 weight/bias gradient
-    (x, grid and the no_grad statistics receive none, as in the reference)."""
+    One kernel writes the trunk layout directly.  Backward is the fc0 weight/bias gradient and, when x or grid
+    requires grad, their gradient from one more kernel (fno_lift_dgrad).  Only the statistics are constants: the
+    reference computes them under no_grad, while the normalisation, the grid concat and fc0 are differentiated, so a
+    prediction fed back as the next input (rollout training) or a loss taken w.r.t. the input field gets its full
+    gradient."""
 
     @staticmethod
     def forward(ctx, x, grid, stats, W0, b0, geo):
@@ -153,14 +156,21 @@ class LiftFn(torch.autograd.Function):
         h = lib.lift_fwd(geo, x, grid, stats, W0, b0)
         ctx.geo = geo
         ctx.w_shape = W0.shape
-        ctx.save_for_backward(x, grid, stats)
+        ctx.in_shapes = (x.shape, grid.shape)
+        need_data = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
+        ctx.save_for_backward(x, grid, stats, W0 if need_data else None)
         return h
 
     @staticmethod
     def backward(ctx, dh):
-        x, grid, stats = ctx.saved_tensors
-        gW0, gb0 = lib.lift_bwd(ctx.geo, x, grid, stats, dh.contiguous(), ctx.w_shape)
-        return None, None, None, gW0, gb0, None
+        x, grid, stats, W0 = ctx.saved_tensors
+        dh = dh.contiguous()
+        gW0, gb0 = lib.lift_bwd(ctx.geo, x, grid, stats, dh, ctx.w_shape)
+        dx = dgrid = None
+        if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
+            dx, dgrid = lib.lift_dgrad(ctx.geo, dh, W0, stats, *ctx.in_shapes, need_dx=ctx.needs_input_grad[0],
+                                       need_dgrid=ctx.needs_input_grad[1])
+        return dx, dgrid, None, gW0, gb0, None
 
 
 class HeadFn(torch.autograd.Function):
@@ -194,6 +204,19 @@ def lift(x, grid, W0, b0, padding: int):
 
 def head(h, W1, b1, W2, b2, stats, geo):
     return HeadFn.apply(h, W1, b1, W2, b2, stats, geo)
+
+
+class WindowShiftFn(torch.autograd.Function):
+    """xx' = cat(xx[..., 1:, :], pred) along the time axis (metrics.py:344) with its adjoint, so that a rollout can be
+    trained through: forward fno_window_shift, backward fno_window_shift_bwd (one launch each)."""
+
+    @staticmethod
+    def forward(ctx, xx, pred):
+        return lib.window_shift(xx.contiguous(), pred.contiguous())
+
+    @staticmethod
+    def backward(ctx, g):
+        return lib.window_shift_bwd(g.contiguous(), need_xx=ctx.needs_input_grad[0], need_pred=ctx.needs_input_grad[1])
 
 
 class SpectralConv1dFn(torch.autograd.Function):

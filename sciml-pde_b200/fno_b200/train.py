@@ -32,6 +32,35 @@ def global_grad_norm(params) -> torch.Tensor:
     return torch.linalg.vector_norm(torch.stack(norms))
 
 
+def rollout_loss(model, xx: torch.Tensor, yy: torch.Tensor, grid: torch.Tensor, steps: int):
+    """Multi-step ("pushforward" / unrolled autoregressive) loss, upstream PDEBench's ``training_type="autoregressive"``:
+    for k < steps, ``pred_k = model(xx_k, grid)``, ``loss_k = nrmse(pred_k, yy[..., k:k+1, :]).mean()`` and
+    ``xx_{k+1} = cat(xx_k[..., 1:, :], pred_k)``, no shift after the last step.  The gradient flows through every fed-back
+    prediction (fno_lift_dgrad, fno_window_shift_bwd).  Returns ``(mean_k loss_k, stacked per-step losses [steps])``.
+
+    The mean, not upstream's sum, so that ``steps=1`` is exactly the single-step loss and the adaptive clip
+    ``max(5, 0.1 * total_norm)`` keeps its scale as ``steps`` grows.
+
+    Torch arithmetic in the step: the mean of the ``steps`` losses and, in the backward, the adds with which autograd sums
+    two gradients into every fed-back prediction (``steps - 1``) and every intermediate window (``steps - 2``).  A
+    target frame ``yy[..., k:k+1, :]`` that is not contiguous is copied before the fused loss reads it."""
+    from . import lib, ops
+    from .steptail import nrmse_loss
+
+    if steps < 1:
+        raise lib.FnoError(f"rollout_loss: steps must be >= 1, got {steps}")
+    if yy.shape[-2] < steps:
+        raise lib.FnoError(f"rollout_loss: yy has {yy.shape[-2]} target frames, {steps} rollout steps need {steps}")
+    losses = []
+    for k in range(steps):
+        pred = model(xx, grid)
+        losses.append(nrmse_loss(pred, yy[..., k:k + 1, :]))
+        if k + 1 < steps:
+            xx = ops.WindowShiftFn.apply(xx, pred)
+    per_step = torch.stack(losses)
+    return per_step.mean(), per_step
+
+
 class TrainStep:
     """One optimisation step of FNO2d/FNO3d (``aux=False``) or the two-head joint model."""
 
@@ -94,14 +123,24 @@ class FusedTrainStep:
     and refills them between steps; other inputs fall back to the copying graph.  Under data
     parallelism (``dp``) the optimizer reads the reduced bucket views in place (``own_grads=False``); with
     ``graph=True`` the step is two graph replays around the bucket all-reduces (issued in ``dp.finish()`` on the same
-    stream); without it they are issued from autograd hooks and overlap the rest of the backward pass."""
+    stream); without it they are issued from autograd hooks and overlap the rest of the backward pass.
+
+    ``rollout_steps=K > 1`` trains on the K-step rollout loss (``rollout_loss``): ``yy`` carries at least K target frames
+    and the step returns the K per-step losses.  Eager, graph and ``alias_inputs`` steps work as for K = 1; the two-head
+    joint loss (``auxiliary_weight``) has no rollout form."""
 
     def __init__(self, model, lr: float = 1e-3, weight_decay: float = 1e-4, t_max: float = 0.0, betas=(0.9, 0.999),
                  eps: float = 1e-8, dp: Optional[BucketedGradAllReduce] = None, graph: bool = False,
                  auxiliary_weight: Optional[float] = None, alias_inputs: bool = False, max_graphs: int = 2,
-                 param_groups=None):
+                 param_groups=None, rollout_steps: int = 1):
+        from . import lib
         from .steptail import FusedClipAdam
 
+        if rollout_steps < 1:
+            raise lib.FnoError(f"FusedTrainStep: rollout_steps must be >= 1, got {rollout_steps}")
+        if rollout_steps > 1 and auxiliary_weight is not None:
+            raise lib.FnoError("FusedTrainStep: the two-head joint loss (auxiliary_weight) has no rollout form")
+        self.rollout_steps = rollout_steps
         self.model = model
         self.dp = dp
         self.aux_w = auxiliary_weight
@@ -123,7 +162,10 @@ class FusedTrainStep:
     def _fwd_bwd(self, *batch, weight=None):
         from .steptail import nrmse_loss
 
-        if self.aux_w is None:
+        if self.rollout_steps > 1:
+            xx, yy, grid = batch
+            loss, ret = rollout_loss(self.model, xx, yy, grid, self.rollout_steps)
+        elif self.aux_w is None:
             xx, yy, grid = batch
             loss = nrmse_loss(self.model(xx, grid), yy)
             ret = loss
@@ -172,6 +214,10 @@ class FusedTrainStep:
 
     def __call__(self, *batch, weight=None):
         """``weight`` (data parallelism, eager only): see TrainStep.__call__."""
+        if self.rollout_steps > 1 and batch[1].shape[-2] < self.rollout_steps:
+            from . import lib
+            raise lib.FnoError(f"FusedTrainStep: yy has {batch[1].shape[-2]} target frames, rollout_steps="
+                               f"{self.rollout_steps} needs {self.rollout_steps}")
         if not self.use_graph:
             return self._eager(*batch, weight=weight)
         if weight is not None:
