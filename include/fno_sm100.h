@@ -294,6 +294,18 @@ int fno_window_shift(const float* xx, const float* pred, float* xx_out, long poi
  * Either output may be NULL (not both); gxx != g.                                                   */
 int fno_window_shift_bwd(const float* g, float* gxx, float* gpred, long points, int T0, int V,
                          fno_stream_t stream);
+/* The same shift over the two-head model's joined window xx [points, T0, V] (primary points first,
+ * then auxiliary ones): point p takes its new last frame from pred_a [points_a, 1, V] when
+ * p < points_a and from pred_b [points - points_a, 1, V] otherwise, so that both streams are fed
+ * back without splitting or re-joining the window.  0 <= points_a <= points; pred_a (pred_b) may be
+ * NULL when points_a == 0 (== points); xx_out aliases no input.  fno_window_shift is the
+ * points_a == points case of the same kernel.                                                      */
+int fno_window_shift_split(const float* xx, const float* pred_a, const float* pred_b, float* xx_out,
+                           long points_a, long points, int T0, int V, fno_stream_t stream);
+/* Its adjoint: gxx as for fno_window_shift_bwd, gpred_a / gpred_b = g[.., T0-1, :] of their points.
+ * Any output may be NULL (not all of them); no output aliases g.                                   */
+int fno_window_shift_split_bwd(const float* g, float* gxx, float* gpred_a, float* gpred_b,
+                               long points_a, long points, int T0, int V, fno_stream_t stream);
 
 /* ---- step tail: loss, gradient clipping, Adam, LR schedule (SURVEY 8f row f3) --------------------- */
 /* nrmse(out, target).mean() of fno/train.py:34-40,:266-267 for out / target [B, P, V] (P = pixels x

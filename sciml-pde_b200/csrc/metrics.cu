@@ -226,29 +226,50 @@ metric_final_kernel(const double* __restrict__ sums, const float* __restrict__ b
 }
 
 // xx_out[..., t, :] = xx[..., t + 1, :] (t < T0 - 1),  xx_out[..., T0 - 1, :] = pred[..., 0, :]   (metrics.py:344)
+// over a window whose first points_a points take their new frame from pred_a and the rest from pred_b (the joint
+// model's primary and auxiliary rows); the single-stream shift is points_a = points
 __global__ void __launch_bounds__(256)
-window_shift_kernel(const float* __restrict__ xx, const float* __restrict__ pred, float* __restrict__ out, long points,
-                    int T0, int V) {
+window_shift_kernel(const float* __restrict__ xx, const float* __restrict__ pred_a, const float* __restrict__ pred_b,
+                    float* __restrict__ out, long points_a, long points, int T0, int V) {
   const long total = points * T0 * V;
   const int TV = T0 * V;
-  for (long o = (long)blockIdx.x * blockDim.x + threadIdx.x; o < total; o += (long)gridDim.x * blockDim.x) {
-    const long pt = o / TV;
-    const int e = (int)(o - pt * TV);
-    out[o] = (e < TV - V) ? __ldg(xx + o + V) : __ldg(pred + pt * V + (e - (TV - V)));
+  // (point, offset in the point) of o, advanced by the grid stride without a 64-bit division per element
+  const long stride = (long)gridDim.x * blockDim.x, sp = stride / TV;
+  const int se = (int)(stride - sp * TV);
+  long o = (long)blockIdx.x * blockDim.x + threadIdx.x, pt = o / TV;
+  int e = (int)(o - pt * TV);
+  for (; o < total; o += stride) {
+    const int v = e - (TV - V);
+    const float* src = v < 0 ? xx + o + V : pt < points_a ? pred_a + pt * V + v : pred_b + (pt - points_a) * V + v;
+    out[o] = __ldg(src);
+    pt += sp;
+    e += se;
+    if (e >= TV) { e -= TV; ++pt; }
   }
 }
 
-// its adjoint: gxx[..., 0, :] = 0, gxx[..., t, :] = g[..., t - 1, :], gpred = g[..., T0 - 1, :] (either output may be null)
+// its adjoint: gxx[..., 0, :] = 0, gxx[..., t, :] = g[..., t - 1, :], gpred_a / gpred_b = g[..., T0 - 1, :] of their
+// points (any output may be null)
 __global__ void __launch_bounds__(256)
-window_shift_bwd_kernel(const float* __restrict__ g, float* __restrict__ gxx, float* __restrict__ gpred, long points,
-                        int T0, int V) {
+window_shift_bwd_kernel(const float* __restrict__ g, float* __restrict__ gxx, float* __restrict__ gpred_a,
+                        float* __restrict__ gpred_b, long points_a, long points, int T0, int V) {
   const long total = points * T0 * V;
   const int TV = T0 * V;
-  for (long o = (long)blockIdx.x * blockDim.x + threadIdx.x; o < total; o += (long)gridDim.x * blockDim.x) {
-    const long pt = o / TV;
-    const int e = (int)(o - pt * TV);
+  const long stride = (long)gridDim.x * blockDim.x, sp = stride / TV;
+  const int se = (int)(stride - sp * TV);
+  long o = (long)blockIdx.x * blockDim.x + threadIdx.x, pt = o / TV;
+  int e = (int)(o - pt * TV);
+  for (; o < total; o += stride) {
     if (gxx != nullptr) gxx[o] = e < V ? 0.f : __ldg(g + o - V);
-    if (gpred != nullptr && e >= TV - V) gpred[pt * V + (e - (TV - V))] = __ldg(g + o);
+    const int v = e - (TV - V);
+    if (v >= 0) {
+      float* dst = pt < points_a ? (gpred_a != nullptr ? gpred_a + pt * V + v : nullptr)
+                                 : (gpred_b != nullptr ? gpred_b + (pt - points_a) * V + v : nullptr);
+      if (dst != nullptr) *dst = __ldg(g + o);
+    }
+    pt += sp;
+    e += se;
+    if (e >= TV) { e -= TV; ++pt; }
   }
 }
 
@@ -355,26 +376,54 @@ extern "C" int fno_metric_func(const float* pred, const float* target, void* wor
   return check_launch("metric_final_kernel");
 }
 
-extern "C" int fno_window_shift(const float* xx, const float* pred, float* xx_out, long points, int T0, int V,
-                                fno_stream_t stream) {
-  if (!xx || !pred || !xx_out || points <= 0 || T0 <= 0 || V <= 0 || xx == xx_out) {
-    set_error("fno_window_shift: bad argument (in-place shift is not supported)");
+namespace {
+int window_shift_impl(const char* name, const float* xx, const float* pred_a, const float* pred_b, float* xx_out,
+                      long points_a, long points, int T0, int V, cudaStream_t st) {
+  if (!xx || !xx_out || points <= 0 || T0 <= 0 || V <= 0 || points_a < 0 || points_a > points ||
+      (points_a > 0 && !pred_a) || (points_a < points && !pred_b) || xx_out == xx || xx_out == pred_a ||
+      xx_out == pred_b) {
+    set_error("%s: bad argument (0 <= points_a <= points, a prediction for every point; in-place shift is not "
+              "supported)", name);
     return FNO_E_ARG;
   }
-  window_shift_kernel<<<grid_for(points * T0 * V), 256, 0, static_cast<cudaStream_t>(stream)>>>(xx, pred, xx_out, points,
-                                                                                              T0, V);
+  window_shift_kernel<<<grid_for(points * T0 * V), 256, 0, st>>>(xx, pred_a, pred_b, xx_out, points_a, points, T0, V);
   count_launch();
   return check_launch("window_shift_kernel");
 }
 
-extern "C" int fno_window_shift_bwd(const float* g, float* gxx, float* gpred, long points, int T0, int V,
-                                    fno_stream_t stream) {
-  if (!g || (!gxx && !gpred) || points <= 0 || T0 <= 0 || V <= 0 || g == gxx) {
-    set_error("fno_window_shift_bwd: bad argument (need gxx or gpred; in-place is not supported)");
+int window_shift_bwd_impl(const char* name, const float* g, float* gxx, float* gpred_a, float* gpred_b, long points_a,
+                          long points, int T0, int V, cudaStream_t st) {
+  if (!g || (!gxx && !gpred_a && !gpred_b) || points <= 0 || T0 <= 0 || V <= 0 || points_a < 0 || points_a > points ||
+      g == gxx || g == gpred_a || g == gpred_b) {
+    set_error("%s: bad argument (need an output, 0 <= points_a <= points; in-place is not supported)", name);
     return FNO_E_ARG;
   }
-  window_shift_bwd_kernel<<<grid_for(points * T0 * V), 256, 0, static_cast<cudaStream_t>(stream)>>>(g, gxx, gpred,
-                                                                                                    points, T0, V);
+  window_shift_bwd_kernel<<<grid_for(points * T0 * V), 256, 0, st>>>(g, gxx, gpred_a, gpred_b, points_a, points, T0, V);
   count_launch();
   return check_launch("window_shift_bwd_kernel");
+}
+}  // namespace
+
+extern "C" int fno_window_shift(const float* xx, const float* pred, float* xx_out, long points, int T0, int V,
+                                fno_stream_t stream) {
+  return window_shift_impl("fno_window_shift", xx, pred, nullptr, xx_out, points, points, T0, V,
+                           static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int fno_window_shift_bwd(const float* g, float* gxx, float* gpred, long points, int T0, int V,
+                                    fno_stream_t stream) {
+  return window_shift_bwd_impl("fno_window_shift_bwd", g, gxx, gpred, nullptr, points, points, T0, V,
+                               static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int fno_window_shift_split(const float* xx, const float* pred_a, const float* pred_b, float* xx_out,
+                                      long points_a, long points, int T0, int V, fno_stream_t stream) {
+  return window_shift_impl("fno_window_shift_split", xx, pred_a, pred_b, xx_out, points_a, points, T0, V,
+                           static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int fno_window_shift_split_bwd(const float* g, float* gxx, float* gpred_a, float* gpred_b, long points_a,
+                                          long points, int T0, int V, fno_stream_t stream) {
+  return window_shift_bwd_impl("fno_window_shift_split_bwd", g, gxx, gpred_a, gpred_b, points_a, points, T0, V,
+                               static_cast<cudaStream_t>(stream));
 }

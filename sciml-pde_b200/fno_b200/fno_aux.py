@@ -14,6 +14,7 @@ import torch
 from torch import nn
 
 from . import fno as _base
+from . import ops
 
 
 class FNO2d(_base.FNO2d):
@@ -52,9 +53,15 @@ class FNO3d(_base.FNO3d):
 
 def _two_head_forward(model, x, grid, x_aux, grid_aux):
     _base._check_cuda(model, x)
-    nb = x.shape[0]
-    h, stats, geo = _base._lift(model, torch.cat((x, x_aux), dim=0), torch.cat((grid, grid_aux), dim=0))
+    return _joint_forward(model, torch.cat((x, x_aux), dim=0), torch.cat((grid, grid_aux), dim=0), x.shape[0])
+
+
+def _joint_forward(model, xj, gridj, nb):
+    """The joint forward on an already joined window xj = cat(x, x_aux), gridj = cat(grid, grid_aux); rows [0, nb) are
+    the primary stream.  A rollout joins once and feeds both predictions back into xj (ops.JointWindowShiftFn)."""
+    h, stats, geo = _base._lift(model, xj, gridj)
     h = _base._trunk(model, h)
-    out_p = _base._project(model, h[:nb], model.fc2_primary, stats[:nb].contiguous(), geo)
-    out_a = _base._project(model, h[nb:], model.fc2_auxiliary, stats[nb:].contiguous(), geo)
-    return out_p, out_a
+    out_p, out_a = ops.TwoHeadFn.apply(h, model.fc1.weight, model.fc1.bias, model.fc2_primary.weight,
+                                       model.fc2_primary.bias, model.fc2_auxiliary.weight, model.fc2_auxiliary.bias,
+                                       stats, geo, nb)
+    return out_p.unsqueeze(-2), out_a.unsqueeze(-2)

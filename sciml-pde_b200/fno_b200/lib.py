@@ -62,6 +62,8 @@ def load():
             "fno_metric_func": (i, [vp, vp, vp, vp, i, i, i, i, i, i, f, f, f, i, i, vp]),
             "fno_window_shift": (i, [vp, vp, vp, l, i, i, vp]),
             "fno_window_shift_bwd": (i, [vp, vp, vp, l, i, i, vp]),
+            "fno_window_shift_split": (i, [vp, vp, vp, vp, l, l, i, i, vp]),
+            "fno_window_shift_split_bwd": (i, [vp, vp, vp, vp, l, l, i, i, vp]),
             "fno_set_math_mode": (i, [i]),
             "fno_get_math_mode": (i, []),
             "fno_plan_destroy": (i, [vp]),
@@ -131,6 +133,7 @@ EXPORTED_SYMBOLS = (
     "fno_nrmse_workspace_bytes", "fno_nrmse_fwd", "fno_nrmse_bwd", "fno_opt_chunk_floats",
     "fno_opt_chunk_bytes", "fno_clip_adam_step",
     "fno_metric_workspace_bytes", "fno_metric_func", "fno_window_shift", "fno_window_shift_bwd",
+    "fno_window_shift_split", "fno_window_shift_split_bwd",
     "fno_sc1d_fwd_transform", "fno_sc1d_inv_transform", "fno_mix1d_fwd", "fno_mix1d_bwd",
 )
 
@@ -612,11 +615,17 @@ def head_fwd(geo: TrunkGeo, h, W1, b1, W2, b2, stats) -> torch.Tensor:
 
 
 @_on_tensor_device
-def head_bwd(geo: TrunkGeo, h, dout, W1, b1, W2, stats):
+def head_bwd(geo: TrunkGeo, h, dout, W1, b1, W2, stats, dh_out: Optional[torch.Tensor] = None):
+    """Returns (dh, gW1, gb1, gW2, gb2).  ``dh_out``: where to write dh (shape of h, e.g. this head's sample range of
+    a larger trunk gradient); every form writes it whole, zero in the padding."""
     _require(dout, torch.float32, "dout")
     B, C, HID, V = h.shape[0], h.shape[1], W1.shape[0], W2.shape[0]
     lib = load()
-    dh = torch.empty_like(h)
+    if dh_out is not None:
+        _require(dh_out, torch.float32, "dh_out")
+        if dh_out.shape != h.shape:
+            raise FnoError(f"head_bwd: dh_out {tuple(dh_out.shape)} must have the shape of h {tuple(h.shape)}")
+    dh = torch.empty_like(h) if dh_out is None else dh_out
     gW1, gb1 = torch.empty_like(W1), torch.empty(HID, dtype=torch.float32, device=h.device)
     gW2, gb2 = torch.empty_like(W2), torch.empty(V, dtype=torch.float32, device=h.device)
     tc = HEAD_BWD_TC and HID == 128 and C <= 23 and V <= 8
@@ -708,6 +717,49 @@ def window_shift_bwd(g: torch.Tensor, *, need_xx: bool = True, need_pred: bool =
     _check(load().fno_window_shift_bwd(g.data_ptr(), _ptr(gxx), _ptr(gpred), g.numel() // (T0 * V), T0, V, _stream()),
            "fno_window_shift_bwd")
     return gxx, gpred
+
+
+@_on_tensor_device
+def window_shift_split(xx: torch.Tensor, pred_a: torch.Tensor, pred_b: torch.Tensor) -> torch.Tensor:
+    """Joined window xx [Na + Nb, *spatial, T0, V] (the rows of pred_a's stream first), pred_a [Na, *spatial, 1, V],
+    pred_b [Nb, *spatial, 1, V] -> cat(xx[..., 1:, :], cat(pred_a, pred_b)) in one kernel, without joining the two
+    predictions."""
+    for t, n in ((xx, "xx"), (pred_a, "pred_a"), (pred_b, "pred_b")):
+        _require(t, torch.float32, n)
+    T0, V = xx.shape[-2:]
+    tail = tuple(xx.shape[1:-2]) + (1, V)
+    if (tuple(pred_a.shape[1:]) != tail or tuple(pred_b.shape[1:]) != tail
+            or pred_a.shape[0] + pred_b.shape[0] != xx.shape[0]):
+        raise FnoError(f"window_shift_split: predictions {tuple(pred_a.shape)} + {tuple(pred_b.shape)} do not fill the "
+                       f"last frame of {tuple(xx.shape)}")
+    out = torch.empty_like(xx)
+    points = xx.numel() // (T0 * V)
+    _check(load().fno_window_shift_split(xx.data_ptr(), pred_a.data_ptr(), pred_b.data_ptr(), out.data_ptr(),
+                                         pred_a.numel() // V, points, T0, V, _stream()), "fno_window_shift_split")
+    return out
+
+
+@_on_tensor_device
+def window_shift_split_bwd(g: torch.Tensor, n_a: int, *, need_xx: bool = True, need_a: bool = True,
+                           need_b: bool = True):
+    """Adjoint of window_shift_split: g [N, *spatial, T0, V] -> (gxx or None, gpred_a [n_a, *spatial, 1, V] or None,
+    gpred_b [N - n_a, *spatial, 1, V] or None)."""
+    _require(g, torch.float32, "g")
+    if not 0 <= n_a <= g.shape[0]:
+        raise FnoError(f"window_shift_split_bwd: n_a = {n_a} outside [0, {g.shape[0]}]")
+    if not (need_xx or need_a or need_b):
+        raise FnoError("window_shift_split_bwd: no output requested")
+    T0, V = g.shape[-2:]
+    tail = tuple(g.shape[1:-2]) + (1, V)
+    gxx = torch.empty_like(g) if need_xx else None
+    ga = torch.empty((n_a,) + tail, dtype=torch.float32, device=g.device) if need_a else None
+    gb = torch.empty((g.shape[0] - n_a,) + tail, dtype=torch.float32, device=g.device) if need_b else None
+    if not any(t is not None and t.numel() > 0 for t in (gxx, ga, gb)):
+        return gxx, ga, gb                   # only the gradient of an empty stream was asked for
+    points = g.numel() // (T0 * V)
+    _check(load().fno_window_shift_split_bwd(g.data_ptr(), _ptr(gxx), _ptr(ga), _ptr(gb), points // g.shape[0] * n_a,
+                                             points, T0, V, _stream()), "fno_window_shift_split_bwd")
+    return gxx, ga, gb
 
 
 # ---- SpectralConv1d ------------------------------------------------------------------------------------------

@@ -194,6 +194,38 @@ class HeadFn(torch.autograd.Function):
         return dh, gW1, gb1, gW2, gb2, None, None
 
 
+class TwoHeadFn(torch.autograd.Function):
+    """The two-head joint model's heads on one trunk activation h [Na + Nb, C, ...] (fno_aux.py:187, 216): samples
+    [0, Na) through fc1 -> fc2_primary, samples [Na, Na + Nb) through fc1 -> fc2_auxiliary.
+
+    The sample ranges of h are contiguous views, so the head kernels read them in place.  Backward writes both heads'
+    dh into one trunk-sized tensor (each head kernel writes its range whole, zero padding included), so no zero-filled
+    full-size gradient per head and no add of the two exist; the shared fc1 gradient is the sum of the two heads'
+    [128, C] contributions."""
+
+    @staticmethod
+    def forward(ctx, h, W1, b1, W2a, b2a, W2b, b2b, stats, geo, na):
+        h = h.contiguous()
+        W1, b1 = W1.contiguous(), b1.contiguous()
+        W2a, b2a, W2b, b2b = W2a.contiguous(), b2a.contiguous(), W2b.contiguous(), b2b.contiguous()
+        out_a = lib.head_fwd(geo, h[:na], W1, b1, W2a, b2a, stats[:na])
+        out_b = lib.head_fwd(geo, h[na:], W1, b1, W2b, b2b, stats[na:])
+        ctx.geo, ctx.na = geo, na
+        ctx.save_for_backward(h, W1, b1, W2a, W2b, stats)
+        return out_a, out_b
+
+    @staticmethod
+    def backward(ctx, dout_a, dout_b):
+        h, W1, b1, W2a, W2b, stats = ctx.saved_tensors
+        geo, na = ctx.geo, ctx.na
+        dh = torch.empty_like(h)
+        _, gW1a, gb1a, gW2a, gb2a = lib.head_bwd(geo, h[:na], dout_a.contiguous(), W1, b1, W2a, stats[:na],
+                                                  dh_out=dh[:na])
+        _, gW1b, gb1b, gW2b, gb2b = lib.head_bwd(geo, h[na:], dout_b.contiguous(), W1, b1, W2b, stats[na:],
+                                                  dh_out=dh[na:])
+        return dh, gW1a + gW1b, gb1a + gb1b, gW2a, gb2a, gW2b, gb2b, None, None, None
+
+
 def lift(x, grid, W0, b0, padding: int):
     """Returns (h in trunk layout, stats [B, 2, V], geometry)."""
     geo = lib.TrunkGeo(x.shape[1:-2], padding)
@@ -217,6 +249,22 @@ class WindowShiftFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         return lib.window_shift_bwd(g.contiguous(), need_xx=ctx.needs_input_grad[0], need_pred=ctx.needs_input_grad[1])
+
+
+class JointWindowShiftFn(torch.autograd.Function):
+    """The rollout shift of the two-head model's joined window xj = cat(xx, xx_aux):
+    cat(xj[..., 1:, :], cat(pred, pred_aux)) with its adjoint, one launch each (fno_window_shift_split(_bwd)).  Both
+    streams are fed back without splitting the window or joining the predictions."""
+
+    @staticmethod
+    def forward(ctx, xj, pred_a, pred_b):
+        ctx.na = pred_a.shape[0]
+        return lib.window_shift_split(xj.contiguous(), pred_a.contiguous(), pred_b.contiguous())
+
+    @staticmethod
+    def backward(ctx, g):
+        need = ctx.needs_input_grad
+        return lib.window_shift_split_bwd(g.contiguous(), ctx.na, need_xx=need[0], need_a=need[1], need_b=need[2])
 
 
 class SpectralConv1dFn(torch.autograd.Function):

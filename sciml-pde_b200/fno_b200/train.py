@@ -61,6 +61,42 @@ def rollout_loss(model, xx: torch.Tensor, yy: torch.Tensor, grid: torch.Tensor, 
     return per_step.mean(), per_step
 
 
+def joint_rollout_loss(model, xx: torch.Tensor, yy: torch.Tensor, grid: torch.Tensor, xx_aux: torch.Tensor,
+                       yy_aux: torch.Tensor, grid_aux: torch.Tensor, steps: int, auxiliary_weight: float):
+    """``rollout_loss`` for the two-head joint model (fno_b200.fno_aux), the auxiliary tensors flattened to
+    ``[B * num_aux, ...]`` as the joint loop has them (fno_train_aux.py:251-256).  For k < steps:
+    ``(p_k, a_k) = model(xx_k, grid, xx_aux_k, grid_aux)``, ``lp_k = nrmse(p_k, yy[..., k:k+1, :]).mean()``,
+    ``la_k = nrmse(a_k, yy_aux[..., k:k+1, :]).mean()``, and both streams are fed back,
+    ``xx_{k+1} = cat(xx_k[..., 1:, :], p_k)``, ``xx_aux_{k+1} = cat(xx_aux_k[..., 1:, :], a_k)``, no shift after the last
+    step.  Returns ``(mean_k (lp_k + auxiliary_weight * la_k), per-step losses [steps, 2] with rows (lp_k, la_k))``;
+    ``steps=1`` is the single-step joint loss ``lp + w * la``.
+
+    The streams are joined once at entry.  After that one shift of the joined window feeds both predictions back
+    (ops.JointWindowShiftFn: one launch forward, one backward), so no step joins or splits the window again."""
+    from . import fno_aux, lib, ops
+    from .fno import _check_cuda
+    from .steptail import nrmse_loss
+
+    if steps < 1:
+        raise lib.FnoError(f"joint_rollout_loss: steps must be >= 1, got {steps}")
+    for t, n in ((yy, "yy"), (yy_aux, "yy_aux")):
+        if t.shape[-2] < steps:
+            raise lib.FnoError(f"joint_rollout_loss: {n} has {t.shape[-2]} target frames, {steps} rollout steps need "
+                               f"{steps}")
+    _check_cuda(model, xx)
+    nb = xx.shape[0]
+    xj, gridj = torch.cat((xx, xx_aux), dim=0), torch.cat((grid, grid_aux), dim=0)
+    lps, las = [], []
+    for k in range(steps):
+        p, a = fno_aux._joint_forward(model, xj, gridj, nb)
+        lps.append(nrmse_loss(p, yy[..., k:k + 1, :]))
+        las.append(nrmse_loss(a, yy_aux[..., k:k + 1, :]))
+        if k + 1 < steps:
+            xj = ops.JointWindowShiftFn.apply(xj, p, a)
+    per_step = torch.stack((torch.stack(lps), torch.stack(las)), dim=1)
+    return (per_step[:, 0] + auxiliary_weight * per_step[:, 1]).mean(), per_step
+
+
 class TrainStep:
     """One optimisation step of FNO2d/FNO3d (``aux=False``) or the two-head joint model."""
 
@@ -126,8 +162,9 @@ class FusedTrainStep:
     stream); without it they are issued from autograd hooks and overlap the rest of the backward pass.
 
     ``rollout_steps=K > 1`` trains on the K-step rollout loss (``rollout_loss``): ``yy`` carries at least K target frames
-    and the step returns the K per-step losses.  Eager, graph and ``alias_inputs`` steps work as for K = 1; the two-head
-    joint loss (``auxiliary_weight``) has no rollout form."""
+    and the step returns the K per-step losses.  With ``auxiliary_weight`` (the two-head joint model) it is
+    ``joint_rollout_loss``: ``yy`` and ``yy_aux`` carry at least K frames and the step returns ``[K, 2]``, rows (primary,
+    auxiliary).  Eager, graph and ``alias_inputs`` steps work as for K = 1."""
 
     def __init__(self, model, lr: float = 1e-3, weight_decay: float = 1e-4, t_max: float = 0.0, betas=(0.9, 0.999),
                  eps: float = 1e-8, dp: Optional[BucketedGradAllReduce] = None, graph: bool = False,
@@ -138,8 +175,9 @@ class FusedTrainStep:
 
         if rollout_steps < 1:
             raise lib.FnoError(f"FusedTrainStep: rollout_steps must be >= 1, got {rollout_steps}")
-        if rollout_steps > 1 and auxiliary_weight is not None:
-            raise lib.FnoError("FusedTrainStep: the two-head joint loss (auxiliary_weight) has no rollout form")
+        if rollout_steps > 1 and auxiliary_weight is not None and not hasattr(model, "fc2_auxiliary"):
+            raise lib.FnoError("FusedTrainStep: a rollout with auxiliary_weight needs the two-head joint model "
+                               "(fno_b200.fno_aux)")
         self.rollout_steps = rollout_steps
         self.model = model
         self.dp = dp
@@ -162,7 +200,9 @@ class FusedTrainStep:
     def _fwd_bwd(self, *batch, weight=None):
         from .steptail import nrmse_loss
 
-        if self.rollout_steps > 1:
+        if self.rollout_steps > 1 and self.aux_w is not None:
+            loss, ret = joint_rollout_loss(self.model, *batch, self.rollout_steps, self.aux_w)
+        elif self.rollout_steps > 1:
             xx, yy, grid = batch
             loss, ret = rollout_loss(self.model, xx, yy, grid, self.rollout_steps)
         elif self.aux_w is None:
@@ -214,10 +254,13 @@ class FusedTrainStep:
 
     def __call__(self, *batch, weight=None):
         """``weight`` (data parallelism, eager only): see TrainStep.__call__."""
-        if self.rollout_steps > 1 and batch[1].shape[-2] < self.rollout_steps:
-            from . import lib
-            raise lib.FnoError(f"FusedTrainStep: yy has {batch[1].shape[-2]} target frames, rollout_steps="
-                               f"{self.rollout_steps} needs {self.rollout_steps}")
+        if self.rollout_steps > 1:
+            targets = ((1, "yy"), (4, "yy_aux")) if self.aux_w is not None else ((1, "yy"),)
+            for i, n in targets:
+                if batch[i].shape[-2] < self.rollout_steps:
+                    from . import lib
+                    raise lib.FnoError(f"FusedTrainStep: {n} has {batch[i].shape[-2]} target frames, rollout_steps="
+                                       f"{self.rollout_steps} needs {self.rollout_steps}")
         if not self.use_graph:
             return self._eager(*batch, weight=weight)
         if weight is not None:
