@@ -256,6 +256,18 @@ int fno_head_bwd_wide_tc(const float* h, const float* dout, const float* W1, con
 int fno_window_gather(const float* traj, const long long* traj_idx, const int* t_start, float* xx,
                       float* yy, int B, long npix, int T, int V, int initial_step, int rollout,
                       fno_stream_t stream);
+/* The two-head joint model's batch (fno_aux/utils_2d_rd.py items, flattened as fno_train_aux.py:251-256 does):
+ * traj_aux [n_traj, A, pixels, T, V] holds the A auxiliary trajectories of each primary trajectory, and one launch writes
+ * the JOINED window the trunk runs on, primary rows first:
+ *   xj [B + B*A, pixels, initial_step, V]: row b = primary window of item b,
+ *                                          row B + b*A + k = window of traj_aux[traj_idx[b], k] at t_start[b]
+ *   yy [B, pixels, rollout, V],  yy_aux [B*A, pixels, rollout, V]: the targets in the same order.
+ * The (item, stream) of an auxiliary row is computed in the kernel.  A = 0 is fno_window_gather (traj_aux, yy_aux may be
+ * NULL).  FNO_E_ARG for A < 0, a NULL traj_aux / yy_aux with A > 0, a window longer than T, element counts >= 2^32 or
+ * more than 65535 rows, and an output that overlaps a store (checked against the extent of its first trajectory). */
+int fno_window_gather_joint(const float* traj, const float* traj_aux, const long long* traj_idx,
+                            const int* t_start, float* xj, float* yy, float* yy_aux, int B, int A,
+                            long npix, int T, int V, int initial_step, int rollout, fno_stream_t stream);
 
 /* ---- SpectralConv1d (named by north_star; the reference tree has no 1-D layer, so this follows the 2-D layer's
  * conventions, fno/fno.py:35-92, one dimension down) ---------------------------------------------------------------- */

@@ -144,8 +144,9 @@ class DeviceWindows:
 
     def __init__(self, traj: torch.Tensor, initial_step: int = 10, rollout: int = 1, device=None,
                  grid_lo: float = -1.0, grid_hi: float = 1.0):
+        name = type(self).__name__
         if traj.dim() < 4:
-            raise ValueError("DeviceWindows: traj must be [n_traj, T, *spatial, V]")
+            raise ValueError(f"{name}: traj must be [n_traj, T, *spatial, V]")
         device = torch.device(device if device is not None else "cuda")
         self.spatial = tuple(traj.shape[2:-1])
         self.nd = len(self.spatial)
@@ -153,14 +154,19 @@ class DeviceWindows:
         self.initial_step, self.rollout = initial_step, rollout
         self.n_windows = self.T - initial_step - rollout + 1
         if self.n_windows <= 0:
-            raise ValueError("DeviceWindows: trajectories shorter than initial_step + rollout")
-        n_traj = traj.shape[0]
-        perm = (0,) + tuple(range(2, 2 + self.nd)) + (1, 2 + self.nd)          # -> [n, *sp, T, V]
-        self.traj = traj.to(device=device, dtype=torch.float32).permute(*perm).contiguous().view(n_traj, -1, self.T, self.V)
+            raise ValueError(f"{name}: trajectories shorter than initial_step + rollout")
+        self.traj = self._store(traj, device)
         lins = [torch.linspace(grid_lo + (grid_hi - grid_lo) / (2 * n), grid_hi - (grid_hi - grid_lo) / (2 * n), n)
                 for n in self.spatial]                                           # cell centres per axis
         self.grid = torch.stack(torch.meshgrid(*lins, indexing="ij"), dim=-1).to(device)
         self.device = device
+
+    def _store(self, traj: torch.Tensor, device) -> torch.Tensor:
+        """[n, *lead, T, *spatial, V] -> the time-inner device store [n, *lead, pixels, T, V]."""
+        lead = traj.dim() - self.nd - 2                                          # 1, or 2 with the auxiliary axis
+        perm = tuple(range(lead)) + tuple(range(lead + 1, lead + 1 + self.nd)) + (lead, lead + 1 + self.nd)
+        store = traj.to(device=device, dtype=torch.float32).permute(*perm).contiguous()
+        return store.view(tuple(traj.shape[:lead]) + (-1, self.T, self.V))
 
     def __len__(self):
         return self.traj.shape[0] * self.n_windows
@@ -172,19 +178,22 @@ class DeviceWindows:
         ts = (items - ti * self.n_windows).to(torch.int32)
         return ti.contiguous().pin_memory(), ts.contiguous().pin_memory()
 
+    def _device_items(self, items):
+        """items (1-D int64, host or device) or the (ti, ts) pair of ``split_items`` -> (ti, ts, B) on the device."""
+        if isinstance(items, tuple):
+            ti, ts = (t.to(self.device, non_blocking=True) for t in items)
+            return ti, ts, ti.numel()
+        items = items.to(device=self.device, dtype=torch.int64)
+        ti = torch.div(items, self.n_windows, rounding_mode="floor").contiguous()
+        ts = (items - ti * self.n_windows).to(torch.int32).contiguous()
+        return ti, ts, items.numel()
+
     def batch(self, items, out=None):
         """items: 1-D int64 (host or device), or the (ti, ts) pair of ``split_items`` -> (xx [B,*sp,T0,V], yy [B,*sp,R,V],
         grid [B,*sp,nd]) on the device.  ``out = (xx, yy)``: gather into caller-owned buffers (fixed addresses)."""
         from . import lib
 
-        if isinstance(items, tuple):
-            ti, ts = (t.to(self.device, non_blocking=True) for t in items)
-            B = ti.numel()
-        else:
-            items = items.to(device=self.device, dtype=torch.int64)
-            ti = torch.div(items, self.n_windows, rounding_mode="floor").contiguous()
-            ts = (items - ti * self.n_windows).to(torch.int32).contiguous()
-            B = items.numel()
+        ti, ts, B = self._device_items(items)
         xx, yy = lib.window_gather(self.traj, ti, ts, self.initial_step, self.rollout, out=out)
         xx = xx.view((B,) + self.spatial + (self.initial_step, self.V))
         yy = yy.view((B,) + self.spatial + (self.rollout, self.V))
@@ -199,6 +208,59 @@ class DeviceWindows:
         step: ``step(xx, yy, grid, weight=w)``) -- required whenever ``len(self) % (batch * world) != 0``."""
         for items, w in epoch_plan(len(self), batch, shuffle, seed, epoch, rank, world):
             if world > 1 and not with_weight and w != 1.0:
-                raise ValueError("DeviceWindows.epoch: ragged global batch under data parallelism -- iterate with "
+                raise ValueError(f"{type(self).__name__}.epoch: ragged global batch under data parallelism -- iterate with "
                                  "with_weight=True and pass the weight to the train step")
             yield (self.batch(items) + (w,)) if with_weight else self.batch(items)
+
+
+class DeviceJointWindows(DeviceWindows):
+    """``DeviceWindows`` for the two-head joint model (fno_b200.fno_aux): each item also carries the windows of its ``A``
+    auxiliary trajectories, as ``fno_aux/utils_2d_rd.py`` yields them (``oracle/ref_datasets.AuxFNODatasetMult``).
+
+    ``traj [n, T, *spatial, V]`` and ``traj_aux [n, A, T, *spatial, V]`` (PDEBench layout; ``traj_aux[i, k]`` is the k-th
+    auxiliary trajectory of trajectory i) are stored once, time-inner, in device memory.  Item ``i`` is window
+    ``i % n_windows`` of trajectory ``i // n_windows`` on every stream.  ``batch`` gathers the primary and auxiliary
+    windows with ONE kernel (fno_window_gather_joint) into one joined buffer ``xj [B + B*A, *spatial, T0, V]``, so
+    ``xx = xj[:B]`` and ``xx_aux = xj[B:]`` (flattened ``[B*A, ...]`` in the joint loop's order, fno_train_aux.py:251-256)
+    reach the joint forward as adjacent views and it runs on ``xj`` without concatenating.  The trunk batch is
+    ``B * (1 + A)``."""
+
+    def __init__(self, traj: torch.Tensor, traj_aux: torch.Tensor, initial_step: int = 10, rollout: int = 1, device=None,
+                 grid_lo: float = -1.0, grid_hi: float = 1.0):
+        super().__init__(traj, initial_step, rollout, device, grid_lo, grid_hi)
+        if traj_aux.dim() != traj.dim() + 1 or traj_aux.shape[1] < 1:
+            raise ValueError(f"DeviceJointWindows: traj_aux must be [n_traj, A >= 1, T, *spatial, V], got "
+                             f"{tuple(traj_aux.shape)}")
+        for what, a, p in (("trajectory count n", traj_aux.shape[0], traj.shape[0]), ("frame count T", traj_aux.shape[2],
+                           self.T), ("spatial shape", tuple(traj_aux.shape[3:-1]), self.spatial),
+                           ("channel count V", traj_aux.shape[-1], self.V)):
+            if a != p:
+                raise ValueError(f"DeviceJointWindows: traj_aux {what} {a} does not match traj's {p}")
+        self.A = traj_aux.shape[1]
+        self.traj_aux = self._store(traj_aux, self.device)
+        self._gridj = None
+
+    def batch(self, items, out=None):
+        """items: as ``DeviceWindows.batch`` -> (xx [B,*sp,T0,V], yy [B,*sp,R,V], grid [B,*sp,nd], xx_aux [B*A,*sp,T0,V],
+        yy_aux [B*A,*sp,R,V], grid_aux [B*A,*sp,nd]) on the device; xx / xx_aux are views of one gathered buffer and
+        grid / grid_aux views of one constant joined grid (built once per batch size).  ``out = (xj, yy, yy_aux)``: gather
+        into caller-owned buffers (fixed addresses, for CUDA-graph steps that alias them)."""
+        from . import lib
+
+        ti, ts, B = self._device_items(items)
+        xj, yy, yy_aux = lib.window_gather_joint(self.traj, self.traj_aux, ti, ts, self.initial_step, self.rollout,
+                                                 out=out)
+        rows = B * (1 + self.A)
+        xj = xj.view((rows,) + self.spatial + (self.initial_step, self.V))
+        yy = yy.view((B,) + self.spatial + (self.rollout, self.V))
+        yy_aux = yy_aux.view((B * self.A,) + self.spatial + (self.rollout, self.V))
+        if self._gridj is None or self._gridj.shape[0] != rows:
+            self._gridj = self.grid.unsqueeze(0).expand(rows, *([-1] * (self.nd + 1))).contiguous()
+        return xj[:B], yy, self._gridj[:B], xj[B:], yy_aux, self._gridj[B:]
+
+    def joined_buffers(self, batch: int):
+        """Freshly allocated ``out=`` buffers (xj, yy, yy_aux) for batches of ``batch`` items."""
+        rows, sp = batch * (1 + self.A), self.spatial
+        return (torch.empty((rows,) + sp + (self.initial_step, self.V), device=self.device),
+                torch.empty((batch,) + sp + (self.rollout, self.V), device=self.device),
+                torch.empty((batch * self.A,) + sp + (self.rollout, self.V), device=self.device))

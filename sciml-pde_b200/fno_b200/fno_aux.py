@@ -6,7 +6,8 @@ Differences from fno_b200.fno: ``fc2`` is replaced by ``fc2_primary`` / ``fc2_au
 state_dict keys the reference has), and ``forward(x, grid, x_aux, grid_aux)`` returns
 ``(out_primary, out_auxiliary)``.  The reference runs the shared trunk twice, once per stream;
 no op in the trunk couples samples, so here both streams go through ONE batched pass over
-``cat([x, x_aux])`` -- half the kernel launches, identical results per sample.
+``cat([x, x_aux])`` -- half the kernel launches, identical results per sample.  When ``x_aux`` continues ``x`` in
+memory (``fno_b200.data.DeviceJointWindows`` gathers them so) that joined window is a view and nothing is copied.
 """
 from __future__ import annotations
 
@@ -51,9 +52,26 @@ class FNO3d(_base.FNO3d):
         return _two_head_forward(self, x, grid, x_aux, grid_aux)
 
 
+def is_joined(a: torch.Tensor, b: torch.Tensor) -> bool:
+    """True when ``b`` continues ``a`` in the same storage (both contiguous, neither requiring grad), so that
+    ``cat((a, b))`` is a view, e.g. ``xx`` / ``xx_aux`` from ``fno_b200.data.DeviceJointWindows``."""
+    return (not a.requires_grad and not b.requires_grad and a.is_contiguous() and b.is_contiguous()
+            and a.dtype == b.dtype and a.device == b.device and a.dim() == b.dim() and a.shape[1:] == b.shape[1:]
+            and a.untyped_storage().data_ptr() == b.untyped_storage().data_ptr()
+            and b.data_ptr() == a.data_ptr() + a.numel() * a.element_size())
+
+
+def joined(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
+    """``torch.cat((a, b), dim=0)``: the joined view when ``is_joined(a, b)``, no copy; a concatenation otherwise."""
+    if not is_joined(a, b):
+        return torch.cat((a, b), dim=0)
+    shape = (a.shape[0] + b.shape[0],) + tuple(a.shape[1:])
+    return a.as_strided(shape, torch.empty(shape, device="meta").stride(), a.storage_offset())
+
+
 def _two_head_forward(model, x, grid, x_aux, grid_aux):
     _base._check_cuda(model, x)
-    return _joint_forward(model, torch.cat((x, x_aux), dim=0), torch.cat((grid, grid_aux), dim=0), x.shape[0])
+    return _joint_forward(model, joined(x, x_aux), joined(grid, grid_aux), x.shape[0])
 
 
 def _joint_forward(model, xj, gridj, nb):

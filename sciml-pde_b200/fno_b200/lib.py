@@ -54,6 +54,7 @@ def load():
             "fno_plan2d_create": (i, [i, i, i, i, i, vpp]),
             "fno_plan3d_create": (i, [i, i, i, i, i, i, i, vpp]),
             "fno_window_gather": (i, [vp, vp, vp, vp, vp, i, l, i, i, i, i, vp]),
+            "fno_window_gather_joint": (i, [vp, vp, vp, vp, vp, vp, vp, i, i, l, i, i, i, i, vp]),
             "fno_sc1d_fwd_transform": (i, [vp, vp, l, i, i, i, f, vp]),
             "fno_sc1d_inv_transform": (i, [vp, vp, vp, l, i, i, i, f, vp]),
             "fno_mix1d_fwd": (i, [vp, vp, vp, i, i, i, i, vp]),
@@ -120,7 +121,7 @@ K1_TENSOR_CORES = os.environ.get("FNO_K1_TC", "1") != "0"
 
 EXPORTED_SYMBOLS = (
     "fno_version", "fno_sm_arch", "fno_last_error", "fno_launch_count", "fno_shutdown",
-    "fno_set_math_mode", "fno_get_math_mode", "fno_window_gather",
+    "fno_set_math_mode", "fno_get_math_mode", "fno_window_gather", "fno_window_gather_joint",
     "fno_plan2d_create", "fno_plan3d_create", "fno_plan_destroy", "fno_plan_workspace_bytes",
     "fno_sc2d_fwd_transform", "fno_sc2d_fwd_workspace_bytes", "fno_sc2d_fwd_transform_ws",
     "fno_sc3d_fwd_transform", "fno_mix_fwd", "fno_mix_bwd", "fno_mix_tc_supported",
@@ -667,6 +668,46 @@ def window_gather(traj: torch.Tensor, traj_idx: torch.Tensor, t_start: torch.Ten
                                     yy.data_ptr(), B, npix, T, V, initial_step, rollout, _stream()),
            "fno_window_gather")
     return xx, yy
+
+
+def _overlaps(a: torch.Tensor, b: torch.Tensor) -> bool:
+    a0, b0 = a.data_ptr(), b.data_ptr()
+    return a0 < b0 + b.numel() * b.element_size() and b0 < a0 + a.numel() * a.element_size()
+
+
+@_on_tensor_device
+def window_gather_joint(traj: torch.Tensor, traj_aux: torch.Tensor, traj_idx: torch.Tensor, t_start: torch.Tensor,
+                        initial_step: int, rollout: int, out=None):
+    """traj [n, pixels, T, V], traj_aux [n, A, pixels, T, V] (device, time-inner) -> xj [B + B*A, pixels, initial_step, V]
+    (primary rows, then item b's auxiliary stream k at row B + b*A + k), yy [B, pixels, rollout, V],
+    yy_aux [B*A, pixels, rollout, V]; one copy kernel.  ``out = (xj, yy, yy_aux)``: caller-owned buffers."""
+    _require(traj, torch.float32, "traj")
+    _require(traj_aux, torch.float32, "traj_aux")
+    if traj.dim() != 4 or traj_aux.dim() != 5 or traj_idx.dtype != torch.int64 or t_start.dtype != torch.int32 or \
+            traj_idx.device != traj.device or t_start.device != traj.device or traj_aux.device != traj.device or \
+            traj_idx.shape != t_start.shape:
+        raise FnoError("window_gather_joint: traj [n, pixels, T, V] and traj_aux [n, A, pixels, T, V] f32, traj_idx "
+                       "int64 [B], t_start int32 [B], one device")
+    n, npix, T, V = traj.shape
+    if traj_aux.shape[0] != n or tuple(traj_aux.shape[2:]) != (npix, T, V):
+        raise FnoError(f"window_gather_joint: traj_aux {tuple(traj_aux.shape)} does not match traj {tuple(traj.shape)}")
+    A, B = traj_aux.shape[1], traj_idx.numel()
+    shapes = ((B * (1 + A), npix, initial_step, V), (B, npix, rollout, V), (B * A, npix, rollout, V))
+    if out is not None:                      # caller-owned: fixed addresses for CUDA-graph steps that alias them
+        for t, s, name in zip(out, shapes, ("xj", "yy", "yy_aux")):
+            _require(t, torch.float32, name)
+            if t.numel() != s[0] * s[1] * s[2] * s[3]:
+                raise FnoError(f"window_gather_joint: out buffer {name} has {t.numel()} elements, needs {s}")
+            if _overlaps(t, traj) or _overlaps(t, traj_aux):
+                raise FnoError(f"window_gather_joint: out buffer {name} aliases a trajectory store")
+        xj, yy, yy_aux = out
+    else:
+        xj, yy, yy_aux = (torch.empty(s, dtype=torch.float32, device=traj.device) for s in shapes)
+    _check(load().fno_window_gather_joint(traj.data_ptr(), traj_aux.data_ptr(), traj_idx.data_ptr(), t_start.data_ptr(),
+                                          xj.data_ptr(), yy.data_ptr(), yy_aux.data_ptr(), B, A, npix, T, V,
+                                          initial_step, rollout, _stream()),
+           "fno_window_gather_joint")
+    return xj, yy, yy_aux
 
 
 @_on_tensor_device

@@ -71,7 +71,7 @@ def joint_rollout_loss(model, xx: torch.Tensor, yy: torch.Tensor, grid: torch.Te
     step.  Returns ``(mean_k (lp_k + auxiliary_weight * la_k), per-step losses [steps, 2] with rows (lp_k, la_k))``;
     ``steps=1`` is the single-step joint loss ``lp + w * la``.
 
-    The streams are joined once at entry.  After that one shift of the joined window feeds both predictions back
+    The streams are joined once at entry (a view, no copy, when they are adjacent in memory: ``fno_aux.joined``).  After that one shift of the joined window feeds both predictions back
     (ops.JointWindowShiftFn: one launch forward, one backward), so no step joins or splits the window again."""
     from . import fno_aux, lib, ops
     from .fno import _check_cuda
@@ -85,7 +85,7 @@ def joint_rollout_loss(model, xx: torch.Tensor, yy: torch.Tensor, grid: torch.Te
                                f"{steps}")
     _check_cuda(model, xx)
     nb = xx.shape[0]
-    xj, gridj = torch.cat((xx, xx_aux), dim=0), torch.cat((grid, grid_aux), dim=0)
+    xj, gridj = fno_aux.joined(xx, xx_aux), fno_aux.joined(grid, grid_aux)
     lps, las = [], []
     for k in range(steps):
         p, a = fno_aux._joint_forward(model, xj, gridj, nb)
@@ -252,6 +252,21 @@ class FusedTrainStep:
             g2.replay()
         return replay, out
 
+    def _static_inputs(self, batch):
+        """The copying graph's input buffers.  Joint-model inputs that arrive joined (``xx_aux`` continuing ``xx``, or
+        ``grid_aux`` continuing ``grid``, as ``data.DeviceJointWindows`` yields them) get one joined buffer per pair, so
+        the captured forward reads the joined window in place instead of concatenating it in the graph."""
+        from .fno_aux import is_joined
+
+        static = [torch.empty_like(t) for t in batch]
+        if self.aux_w is not None and len(batch) == 6:
+            for i, j in ((0, 3), (2, 5)):
+                if is_joined(batch[i], batch[j]):
+                    whole = torch.empty((batch[i].shape[0] + batch[j].shape[0],) + tuple(batch[i].shape[1:]),
+                                        dtype=batch[i].dtype, device=batch[i].device)
+                    static[i], static[j] = whole[:batch[i].shape[0]], whole[batch[i].shape[0]:]
+        return tuple(static)
+
     def __call__(self, *batch, weight=None):
         """``weight`` (data parallelism, eager only): see TrainStep.__call__."""
         if self.rollout_steps > 1:
@@ -272,7 +287,7 @@ class FusedTrainStep:
             # third call: this batch's step runs eagerly on a side stream (the stream-capture warm-up
             # PyTorch asks for), then the same sequence is captured -- capture records, it does not
             # execute -- and every later call is a graph replay
-            self._static_in = tuple(torch.empty_like(t) for t in batch)
+            self._static_in = self._static_inputs(batch)
             for dst, src in zip(self._static_in, batch):
                 dst.copy_(src)
             side = torch.cuda.Stream()
