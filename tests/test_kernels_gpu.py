@@ -21,6 +21,48 @@ def lib():
     return L
 
 
+@pytest.fixture(autouse=True)
+def fp32_mode(lib):
+    """The math mode is library-global state: every test starts in fp32 mode and leaves it there, even when it fails."""
+    assert lib.get_math_mode() == "fp32"
+    try:
+        yield
+    finally:
+        lib.set_math_mode("fp32")
+
+
+def run_modes(lib, low, fn):
+    """{mode: fn()} for fp32, tf32 and -- when ``low`` is bf16 -- bf16 mode, each on the same inputs."""
+    errs = {}
+    for mode in ("fp32", "tf32", "bf16")[:3 if low == "bf16" else 2]:
+        lib.set_math_mode(mode)
+        errs[mode] = fn()
+        torch.cuda.synchronize()
+    lib.set_math_mode("fp32")
+    return errs
+
+
+def check_mode_errors(errs, low, what, shows_mode=None):
+    """errs[mode]: {result name: rel_err vs fp64}.  Every result is within its mode's bound; the results named in
+    ``shows_mode`` (default: all) are more than 4x less accurate than in fp32 mode -- the mode reached the kernel -- and,
+    in bf16 mode, more than 2x less accurate than in tf32 mode -- bf16 rounding reached it too."""
+    print(f"{what} errors:", {m: {k: f"{v:.2e}" for k, v in e.items()} for m, e in errs.items()})
+    assert max(errs["fp32"].values()) <= TOL, errs["fp32"]
+    assert max(errs[low].values()) < MODE_TOL[low], errs[low]
+    for k in shows_mode or errs[low]:
+        assert errs[low][k] > 4 * errs["fp32"][k], (k, errs)
+        if low == "bf16":
+            assert errs["bf16"][k] > 2 * errs["tf32"][k], (k, errs)
+
+
+def mode_params(names, cases):
+    """(low, *case) parameter sets for tf32 and bf16.  The first case keeps the bare mode as its id; ``names`` label the
+    cases after it."""
+    assert len(names) == len(cases) - 1
+    return [pytest.param(low, *case, id=f"{low}-{names[i - 1]}" if i else low)
+            for i, case in enumerate(cases) for low in ("tf32", "bf16")]
+
+
 def dev(a, dtype=None):
     t = torch.from_numpy(np.ascontiguousarray(a))
     if dtype is not None:
@@ -250,59 +292,61 @@ def test_mix_tensor_core(lib, B, Ci, Co, spatial, modes, tc):
     assert err.max() < 1e-5 * np.abs(Y).max()
 
 
-@pytest.mark.parametrize("low", ["tf32", "bf16"])
-def test_pointwise_tensor_core_math_modes(lib, low):
+@pytest.mark.parametrize("low,B,spatial", mode_params(
+    ["cfg3"], [(2, (66, 66)),
+               (3, (258, 258))]))             # cfg-3 plane: wgrad_tc_kernel<64, 64> with a ragged last slab
+def test_pointwise_tensor_core_math_modes(lib, low, B, spatial):
     """The width-64 bypass kernels (pointwise_tc.cu: product, data gradient, weight gradient) follow the math mode."""
     rng = np.random.default_rng(3)
-    B, C, spatial = 2, 64, (66, 66)
+    C = 64
     a = rng.standard_normal((B, C) + spatial).astype(np.float32)
     w = rng.standard_normal((C, C, 1, 1)).astype(np.float32) / 8
     b = rng.standard_normal(C).astype(np.float32)
     ds = rng.standard_normal((B, C) + spatial).astype(np.float32)
     w2 = w.reshape(C, C).astype(np.float64)
-    refs = (O.pointwise_conv(a, w, b), np.einsum("oi,bo...->bi...", w2, ds.astype(np.float64)),
-            np.einsum("bop,bip->oi", ds.reshape(B, C, -1).astype(np.float64), a.reshape(B, C, -1).astype(np.float64)))
-    errs = {}
-    for mode in (low, "fp32"):
-        prev = lib.set_math_mode(mode)
-        try:
-            out = lib.pointwise_fwd(dev(a), dev(w), dev(b))
-            back = lib.pointwise_fwd(dev(ds), dev(w), None, transpose=True)
-            gw, _ = lib.pointwise_wgrad(dev(ds), dev(a), w.shape)
-            torch.cuda.synchronize()
-        finally:
-            lib.set_math_mode(prev)
-        errs[mode] = [O.rel_err(t.cpu().numpy().reshape(r.shape), r) for t, r in zip((out, back, gw), refs)]
-    assert max(errs["fp32"]) < TOL, errs
-    assert max(errs[low]) < MODE_TOL[low], errs
-    assert min(errs[low]) > 4 * max(errs["fp32"]), errs
+    a2, ds2 = a.reshape(B, C, -1).astype(np.float64), ds.reshape(B, C, -1).astype(np.float64)
+    refs = {"out": O.pointwise_conv(a, w, b), "d a": np.einsum("oi,bo...->bi...", w2, ds.astype(np.float64)),
+            "d W": np.einsum("bop,bip->oi", ds2, a2)}
+    da, dsd, wd, bd = dev(a), dev(ds), dev(w), dev(b)
+
+    def errors():
+        got = {"out": lib.pointwise_fwd(da, wd, bd), "d a": lib.pointwise_fwd(dsd, wd, None, transpose=True),
+               "d W": lib.pointwise_wgrad(dsd, da, w.shape)[0]}
+        return {k: O.rel_err(t.cpu().numpy().reshape(refs[k].shape), refs[k]) for k, t in got.items()}
+
+    check_mode_errors(run_modes(lib, low, errors), low, f"bypass {spatial}")
 
 
-@pytest.mark.parametrize("low", ["tf32", "bf16"])
-def test_mix_tensor_core_math_modes(lib, low):
+MIX_MODE_CASES = [
+    # B, C, spatial, modes
+    (16, 64, (34, 34), (8, 8)),
+    (4, 64, (16, 16, 18), (4, 4, 6)),       # 3-D: four corners, three spatial modes
+    (32, 64, (66, 66), (16, 16)),           # cfg 3 (per-GPU batch 32)
+]
+
+
+@pytest.mark.parametrize("low,B,C,spatial,modes", mode_params(["3d", "cfg3"], MIX_MODE_CASES))
+def test_mix_tensor_core_math_modes(lib, low, B, C, spatial, modes):
     """tf32 / bf16 modes reach K2's tensor-core kernels: single pass, stated bounds 2e-3 / 2e-2, visibly worse than fp32."""
     rng = np.random.default_rng(5)
-    B, C, modes = 16, 64, (8, 8)
-    plan = lib.get_plan(torch.device("cuda", 0), (34, 34), modes)
-    ws = [cplx(rng, (C, C) + modes, scale=0.5) for _ in range(2)]
+    plan = lib.get_plan(torch.device("cuda", 0), spatial, modes)
+    assert lib.mix_tc_supported(plan, C, C)
+    ws = [cplx(rng, (C, C) + modes, scale=0.5) for _ in range(2 if len(spatial) == 2 else 4)]
     X, gY = cplx(rng, (B, C) + plan.spec_shape), cplx(rng, (B, C) + plan.spec_shape)
     wcat = O.cat_corner_weights(ws)
     y_ref = O.mix_fwd(X.astype(np.complex128), wcat)
     gx_ref, gw_ref = O.mix_bwd(X.astype(np.complex128), gY.astype(np.complex128), wcat)
-    errs = {}
-    for mode in (low, "fp32"):
-        prev = lib.set_math_mode(mode)
-        try:
-            Y = lib.mix_fwd(plan, dev(X), [dev(w) for w in ws])
-            gX, gws = lib.mix_bwd(plan, dev(X), dev(gY), [dev(w) for w in ws])
-            torch.cuda.synchronize()
-        finally:
-            lib.set_math_mode(prev)
-        errs[mode] = max(O.rel_err(Y.cpu().numpy(), y_ref), O.rel_err(gX.cpu().numpy(), gx_ref),
-                         max(O.rel_err(g.cpu().numpy(), r) for g, r in zip(gws, O.split_corner_grads(gw_ref, 2))))
-    assert errs["fp32"] < TOL, errs
-    assert errs[low] < {"tf32": 2e-3, "bf16": 2e-2}[low], errs
-    assert errs[low] > 4 * errs["fp32"], errs
+    gw_refs = O.split_corner_grads(gw_ref, len(ws))
+    Xd, gYd, wsd = dev(X), dev(gY), [dev(w) for w in ws]
+
+    def errors():
+        Y = lib.mix_fwd(plan, Xd, wsd)
+        gX, gws = lib.mix_bwd(plan, Xd, gYd, wsd)
+        e = {"Y": O.rel_err(Y.cpu().numpy(), y_ref), "d X": O.rel_err(gX.cpu().numpy(), gx_ref)}
+        e.update({f"d W{k}": O.rel_err(g.cpu().numpy(), r) for k, (g, r) in enumerate(zip(gws, gw_refs))})
+        return e
+
+    check_mode_errors(run_modes(lib, low, errors), low, f"K2 {spatial} m {modes}")
 
 
 @pytest.mark.parametrize("B,Co,Ci,spatial", [
@@ -589,13 +633,19 @@ MODE_TOL = {"tf32": TF32_TOL, "bf16": BF16_TOL}
 
 @pytest.mark.parametrize("low", ["tf32", "bf16"])
 @pytest.mark.parametrize("spatial,C,V,B", [((64, 64), 20, 2, 3), ((40, 50), 23, 4, 2),
-                                           ((62, 62), 64, 3, 2)])        # wide trunk: head_wide_tc.cu kernels
+                                           ((62, 62), 64, 3, 2),         # wide trunk: head_wide_tc.cu kernels
+                                           ((64, 64, 64), 20, 5, 1),     # cfg-4 head: 3-D trunk, V = 5
+                                           ((16, 16, 22), 40, 3, 2)])    # 3-D wide trunk: + wgrad_tc_kernel<128, 32>
 def test_head_tf32_mode(lib, spatial, C, V, B, low):
     from fno_b200 import ops
     from oracle import fno_port as P
 
     g = torch.Generator().manual_seed(11)
-    geo = lib.TrunkGeo(spatial, 2)
+    nd = len(spatial)
+    geo = lib.TrunkGeo(spatial, 2 if nd == 2 else 6)
+    narrow = C <= 23
+    wide = bool(lib.load().fno_head_bwd_wide_supported(geo.R_out, geo.Wp, C, 128, V))
+    assert narrow != wide                                   # a tensor-core backward either way
     h = torch.randn((B, C) + geo.padded, generator=g) * 1.5
     W1 = torch.randn(128, C, generator=g) / C ** 0.5
     b1 = torch.randn(128, generator=g) * 0.3
@@ -607,33 +657,25 @@ def test_head_tf32_mode(lib, spatial, C, V, B, low):
     p = {"fc1.weight": W1.double().requires_grad_(), "fc1.bias": b1.double().requires_grad_(),
          "fc2.weight": W2.double().requires_grad_(), "fc2.bias": b2.double().requires_grad_()}
     h64 = h.double().requires_grad_()
-    bshape = (B, 1, 1, V)
-    out_ref = P._project(p, h64, 2, "fc2") * std.double().view(bshape) + mean.double().view(bshape)
+    bshape = (B,) + (1,) * nd + (V,)
+    out_ref = P._project(p, h64, nd, "fc2") * std.double().view(bshape) + mean.double().view(bshape)
     gout = torch.randn(out_ref.shape, generator=g, dtype=torch.float64)
     out_ref.backward(gout)
-    errs = {}
-    for mode in (low, "fp32"):
-        prev = lib.set_math_mode(mode)
-        try:
-            assert lib.get_math_mode() == mode
-            hc = h.cuda().requires_grad_()
-            leaves = [t.cuda().requires_grad_() for t in (W1, b1, W2, b2)]
-            out = ops.head(hc, *leaves, stats.cuda(), geo)
-            out.backward(gout.float().cuda())
-            torch.cuda.synchronize()
-        finally:
-            lib.set_math_mode(prev)
+    names = ("fc1.weight", "fc1.bias", "fc2.weight", "fc2.bias")
+
+    def errors():
+        hc = h.cuda().requires_grad_()
+        leaves = [t.cuda().requires_grad_() for t in (W1, b1, W2, b2)]
+        out = ops.head(hc, *leaves, stats.cuda(), geo)
+        out.backward(gout.float().cuda())
         e = {"out": O.rel_err(out.detach().cpu().numpy(), out_ref.detach().numpy()),
              "dh": O.rel_err(hc.grad.cpu().numpy(), h64.grad.numpy())}
-        for t, name in zip(leaves, ("fc1.weight", "fc1.bias", "fc2.weight", "fc2.bias")):
-            e[name] = O.rel_err(t.grad.cpu().numpy(), p[name].grad.numpy())
-        errs[mode] = e
-    assert lib.get_math_mode() == "fp32"
-    assert max(errs["fp32"].values()) < TOL, errs["fp32"]
-    assert max(errs[low].values()) < MODE_TOL[low], errs[low]
-    # the mode switch is real: a single reduced-precision pass is visibly less accurate than the 3xTF32 split
-    assert errs[low]["out"] > 10 * errs["fp32"]["out"], errs
-    print(f"head {low}-mode errors:", {k: f"{v:.2e}" for k, v in errs[low].items()})
+        e.update({n: O.rel_err(t.grad.cpu().numpy(), p[n].grad.numpy()) for t, n in zip(leaves, names)})
+        return e
+
+    # fc2.bias's gradient is a plain sum of the output gradient: no MMA, the same in every mode
+    check_mode_errors(run_modes(lib, low, errors), low, f"head {spatial} C {C} V {V}",
+                      shows_mode=("out", "dh", "fc1.weight", "fc1.bias", "fc2.weight"))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -657,45 +699,59 @@ def test_device_windows_match_host_windows(lib, spatial, T, V, T0, R):
     assert sorted(seen.tolist()) == list(range(len(ds)))
 
 
-@pytest.mark.parametrize("low", ["tf32", "bf16"])
-def test_fwd_transform_tf32_mode(lib, monkeypatch, low):
+@pytest.mark.parametrize("low,B,C,spatial,modes", mode_params(
+    ["cfg4"], [(4, 20, (130, 130), (12, 12)),
+               (4, 20, (64, 64, 70), (12, 12, 12))]))   # cfg-4 volume: K1's tensor-core stage on the inner planes
+def test_fwd_transform_tf32_mode(lib, monkeypatch, low, B, C, spatial, modes):
     """tf32 / bf16 math modes on the K1 tensor-core kernels (plain and GELU'-premultiply forms): single pass, stated
     bound <= 2e-3 (tf32) / 2e-2 (bf16) relative; fp32 mode (3xTF32) <= 1e-5 on the same inputs."""
     monkeypatch.setattr(lib, "K1_TENSOR_CORES", True)
-    B, C, H, W, m1, m2 = 4, 20, 130, 130, 12, 12
     rng = np.random.default_rng(5)
-    g = rng.standard_normal((B, C, H, W)).astype(np.float32)
-    s_ = (rng.standard_normal((B, C, H, W)) * 1.5).astype(np.float32)
-    plan = lib.get_plan(torch.device("cuda", 0), (H, W), (m1, m2))
-    ref_plain = O.fwd_transform(g, (m1, m2), cmode=0, scale=1.0)
+    shape = (B, C) + spatial
+    g = rng.standard_normal(shape).astype(np.float32)
+    s_ = (rng.standard_normal(shape) * 1.5).astype(np.float32)
+    plan = lib.get_plan(torch.device("cuda", 0), spatial, modes)
+    L = lib.load()
+    if len(spatial) == 2:
+        assert L.fno_sc2d_fwd_workspace_bytes(plan.handle, B * C) > 0
+    else:       # the 3-D workspace carries the W-axis GEMM's scratch only when the inner planes take the tensor cores
+        inner = B * C * spatial[0]
+        assert inner * spatial[1] >= 4096 and L.fno_sc2d_fwd_workspace_bytes(plan.handle, inner) > 0
+        spectra = (8 * B * C * spatial[0] * 2 * modes[1] * modes[2] + 255) // 256 * 256
+        assert L.fno_plan_workspace_bytes(plan.handle, B * C) == spectra + L.fno_sc2d_fwd_workspace_bytes(plan.handle, inner)
+    npix = int(np.prod(spatial))
+    ref_plain = O.fwd_transform(g, modes, cmode=0, scale=1.0)
     ds_ref = g.astype(np.float64) * O.gelu_grad(s_.astype(np.float64))
-    ref_pre = O.fwd_transform(ds_ref, (m1, m2), cmode=1, scale=1.0 / (H * W))
-    errs = {}
-    for mode in (low, "fp32"):
-        prev = lib.set_math_mode(mode)
-        try:
-            X = lib.fwd_transform(plan, dev(g), cmode=0, scale=1.0).cpu().numpy()
-            ds = torch.empty(B, C, H, W, device="cuda")
-            Xp = lib.fwd_transform(plan, dev(g), preact=dev(s_), ds_out=ds, cmode=1, scale=1.0 / (H * W)).cpu().numpy()
-        finally:
-            lib.set_math_mode(prev)
-        errs[mode] = (O.rel_err(X, ref_plain), O.rel_err(Xp, ref_pre), O.rel_err(ds.cpu().numpy(), ds_ref))
-    assert max(errs["fp32"]) < TOL, errs
-    assert max(errs[low][:2]) < MODE_TOL[low], errs
-    assert errs[low][2] < TOL                       # dS itself is computed in fp32 in every mode
-    assert errs[low][0] > 10 * errs["fp32"][0], errs
-    if low == "bf16":
-        assert errs[low][0] > 2 * 3.5e-4, errs       # ... and bf16 is visibly coarser than tf32 (measured 2.9e-4)
-    print(f"K1 {low}-mode errors (plain, premultiply):", f"{errs[low][0]:.2e}", f"{errs[low][1]:.2e}")
+    ref_pre = O.fwd_transform(ds_ref, modes, cmode=1, scale=1.0 / npix)
+    gd, sd = dev(g), dev(s_)
+
+    def errors():
+        X = lib.fwd_transform(plan, gd, cmode=0, scale=1.0)
+        ds = torch.empty_like(gd)
+        Xp = lib.fwd_transform(plan, gd, preact=sd, ds_out=ds, cmode=1, scale=1.0 / npix)
+        return {"plain": O.rel_err(X.cpu().numpy(), ref_plain), "premultiply": O.rel_err(Xp.cpu().numpy(), ref_pre),
+                "dS": O.rel_err(ds.cpu().numpy(), ds_ref)}
+
+    errs = run_modes(lib, low, errors)
+    assert max(e["dS"] for e in errs.values()) <= TOL, errs          # dS itself is computed in fp32 in every mode
+    check_mode_errors(errs, low, f"K1 {spatial}", shows_mode=("plain", "premultiply"))
 
 
-@pytest.mark.parametrize("low", ["tf32", "bf16"])
-def test_fourier_layer_reduced_precision_modes(lib, low):
+LAYER_MODE_CASES = [
+    # B, C, n, m
+    (2, 20, 66, 12),
+    (2, 20, 130, 12),     # cfg-1 plane: 128 lanes + 2 edge columns, K1 on the tensor cores
+    (2, 31, 66, 12),      # widest fused layer (31 channels + the bias column)
+]
+
+
+@pytest.mark.parametrize("low,B,C,n,m", mode_params(["cfg1", "width31"], LAYER_MODE_CASES))
+def test_fourier_layer_reduced_precision_modes(lib, low, B, C, n, m):
     """One whole Fourier layer (K1 -> K2 -> fused tcgen05 K3 + bypass + GELU, forward and backward) in tf32 / bf16 mode
     against the fp64 oracle: stated bounds 2e-3 / 2e-2; fp32 mode <= 1e-5 on the same inputs."""
     from fno_b200 import ops
 
-    B, C, n, m = 2, 20, 66, 12
+    assert lib.layer_fused_supported(lib.get_plan(torch.device("cuda", 0), (n, n), (m, m)), C)
     rng = np.random.default_rng(21)
     a = rng.standard_normal((B, C, n, n)).astype(np.float32)
     wl = (rng.standard_normal((C, C, 1, 1)) / C ** 0.5).astype(np.float32)
@@ -703,25 +759,98 @@ def test_fourier_layer_reduced_precision_modes(lib, low):
     ws = [((rng.random((C, C, m, m)) + 1j * rng.random((C, C, m, m))) / C).astype(np.complex64) for _ in range(2)]
     g = rng.standard_normal((B, C, n, n)).astype(np.float32)
     ref, _ = O.fourier_layer_forward(a, ws, wl, bl, True)
-    gref = O.fourier_layer_backward(a, ws, wl, bl, True, g)
-    errs = {}
-    for mode in (low, "fp32"):
-        prev = lib.set_math_mode(mode)
-        try:
-            ad = dev(a).requires_grad_()
-            wld, bld = dev(wl).requires_grad_(), dev(bl).requires_grad_()
-            wsd = [dev(w).requires_grad_() for w in ws]
-            out = ops.fourier_layer(ad, wld, bld, True, wsd)
-            out.backward(dev(g))
-            torch.cuda.synchronize()
-        finally:
-            lib.set_math_mode(prev)
-        errs[mode] = (O.rel_err(out.detach().cpu().numpy(), ref), O.rel_err(ad.grad.cpu().numpy(), gref[0]),
-                      O.rel_err(wsd[0].grad.cpu().numpy(), gref[1][0]))
-    assert max(errs["fp32"]) < TOL, errs
-    assert max(errs[low]) < MODE_TOL[low], errs
-    assert errs[low][0] > 10 * errs["fp32"][0], errs
-    print(f"Fourier layer {low}-mode errors (out, d input, d spectral weight):", [f"{e:.2e}" for e in errs[low]])
+    ga, gws, gwl, gbl = O.fourier_layer_backward(a, ws, wl, bl, True, g)
+
+    def errors():
+        ad = dev(a).requires_grad_()
+        wld, bld = dev(wl).requires_grad_(), dev(bl).requires_grad_()
+        wsd = [dev(w).requires_grad_() for w in ws]
+        out = ops.fourier_layer(ad, wld, bld, True, wsd)
+        out.backward(dev(g))
+        got = {"out": (out.detach(), ref), "d a": (ad.grad, ga), "d W0": (wsd[0].grad, gws[0]),
+               "d W1": (wsd[1].grad, gws[1]), "d Wl": (wld.grad, gwl), "d bias": (bld.grad, gbl)}
+        return {k: O.rel_err(t.cpu().numpy().reshape(np.shape(r)), r) for k, (t, r) in got.items()}
+
+    check_mode_errors(run_modes(lib, low, errors), low, f"Fourier layer B {B} C {C} n {n} m {m}")
+
+
+def _k1_fp32_form(lib, rng, B, C, H, W):
+    plan = lib.get_plan(torch.device("cuda", 0), (H, W), (12, 12))
+    g, s = dev(rng.standard_normal((B, C, H, W)).astype(np.float32)), dev(rng.standard_normal((B, C, H, W)).astype(np.float32))
+
+    def run():
+        ds = torch.empty_like(g)
+        return lib.fwd_transform(plan, g), lib.fwd_transform(plan, g, preact=s, ds_out=ds, cmode=1, scale=0.1), ds
+    return run
+
+
+def _k2_fp32_form(lib, rng, B, C, spatial, modes):
+    plan = lib.get_plan(torch.device("cuda", 0), spatial, modes)
+    assert not lib.mix_tc_supported(plan, C, C)
+    ws = [dev(cplx(rng, (C, C) + modes)) for _ in range(2)]
+    X, gY = dev(cplx(rng, (B, C) + plan.spec_shape)), dev(cplx(rng, (B, C) + plan.spec_shape))
+
+    def run():
+        gX, gws = lib.mix_bwd(plan, X, gY, ws)
+        return [lib.mix_fwd(plan, X, ws), gX] + gws
+    return run
+
+
+def _bypass_fp32_form(lib, rng, B, C, spatial):
+    a, ds = (dev(rng.standard_normal((B, C) + spatial).astype(np.float32)) for _ in range(2))
+    w, b = dev(rng.standard_normal((C, C, 1, 1)).astype(np.float32)), dev(rng.standard_normal(C).astype(np.float32))
+    return lambda: (lib.pointwise_fwd(a, w, b), lib.pointwise_fwd(ds, w, None, transpose=True),
+                    *lib.pointwise_wgrad(ds, a, w.shape), *lib.pointwise_bwd(ds, a, w))
+
+
+def _head_fp32_form(lib, rng, spatial, C, V, B, fwd):
+    geo = lib.TrunkGeo(spatial, 2 if len(spatial) == 2 else 6)
+    h = dev(rng.standard_normal((B, C) + geo.padded).astype(np.float32))
+    W1, b1 = dev(rng.standard_normal((128, C)).astype(np.float32) / C ** 0.5), dev(rng.standard_normal(128).astype(np.float32))
+    W2, b2 = dev(rng.standard_normal((V, 128)).astype(np.float32) / 11), dev(rng.standard_normal(V).astype(np.float32))
+    stats = dev(np.stack((rng.standard_normal((B, V)), rng.random((B, V)) + 0.5), axis=1).astype(np.float32))
+    dout = dev(rng.standard_normal((B,) + geo.spatial + (V,)).astype(np.float32))
+    return lambda: ((lib.head_fwd(geo, h, W1, b1, W2, b2, stats),) if fwd else ()) + \
+        lib.head_bwd(geo, h, dout, W1, b1, W2, stats)
+
+
+def _inv_epilogue_form(lib, rng, B, C, H, W):
+    plan = lib.get_plan(torch.device("cuda", 0), (H, W), (12, 12))
+    Y, add = dev(cplx(rng, (B, C, 24, 12))), dev(rng.standard_normal((B, C, H, W)).astype(np.float32))
+
+    def run():
+        s_out = torch.empty_like(add)
+        return lib.inv_transform(plan, Y, addend=add, s_out=s_out, apply_gelu=True), s_out
+    return run
+
+
+FP32_FORMS = {
+    "k1_below_envelope": lambda lib, rng: _k1_fp32_form(lib, rng, 1, 20, 130, 130),     # planes * H = 2600 < 4096
+    "k1_odd_w": lambda lib, rng: _k1_fp32_form(lib, rng, 2, 20, 130, 129),
+    "k2_width20": lambda lib, rng: _k2_fp32_form(lib, rng, 4, 20, (34, 34), (12, 12)),
+    "k2_odd_modes": lambda lib, rng: _k2_fp32_form(lib, rng, 3, 64, (40, 40), (4, 5)),
+    "bypass_width20": lambda lib, rng: _bypass_fp32_form(lib, rng, 2, 20, (130, 130)),
+    "head_bwd_fp32": lambda lib, rng: _head_fp32_form(lib, rng, (64, 64), 20, 2, 2, fwd=False),
+    "head_outside_envelopes": lambda lib, rng: _head_fp32_form(lib, rng, (12, 10), 40, 5, 2, fwd=True),
+    "inv_fused_epilogue": lambda lib, rng: _inv_epilogue_form(lib, rng, 2, 20, 130, 130),
+}
+
+
+@pytest.mark.parametrize("form", list(FP32_FORMS))
+def test_fp32_forms_ignore_math_mode(lib, monkeypatch, form):
+    """Kernels that run in FP32 -- shapes outside a tensor-core envelope, or files that have no tensor-core form -- give
+    bitwise the same results in all three math modes: only a tensor-core launch may read the mode."""
+    monkeypatch.setattr(lib, "K1_TENSOR_CORES", True)
+    monkeypatch.setattr(lib, "HEAD_BWD_TC", form != "head_bwd_fp32")
+    run = FP32_FORMS[form](lib, np.random.default_rng(31))
+    results = {}
+    for mode in ("fp32", "tf32", "bf16"):
+        lib.set_math_mode(mode)
+        results[mode] = [t.clone() for t in run() if t is not None]
+        torch.cuda.synchronize()
+    for mode in ("tf32", "bf16"):
+        for k, (a, b) in enumerate(zip(results["fp32"], results[mode])):
+            assert torch.equal(a, b), (mode, k)
 
 
 def test_new_entry_points_reject_bad_arguments(lib):
